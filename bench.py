@@ -7,6 +7,7 @@
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on the host cores
     python bench.py --workload c3|c4|c5 ...   # the other BASELINE.json configurations (one JSON line each)
+    python bench.py ... --dump-outputs DIR    # c2: also write the last timed step's outputs as DIR/<name>.npy
 
 A step = one pass of the hot path over one batch of `--images-per-step` synthetic images per GPU (weak scaling).
 Rank 0 prints ONE JSON line. `value` is timed with the uint8 images already resident in HBM; `e2e` goes through
@@ -74,7 +75,14 @@ def parse():
     ap.add_argument("--no-as-shipped", action="store_true", help="skip the eager-GPU-ViT + CPU-eigsh baseline")
     ap.add_argument("--ref-images-per-step", type=int, default=0, help="0 = 2 x worker processes")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c2: write what the last timed step computed (rank 0) as DIR/<name>.npy, at most 64 MB")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs is implemented for --impl ours --workload c2")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -511,6 +519,34 @@ def load_traffic():
 
 
 # ---------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, evals, evecs, info, feats, feature_images=16, budget=64_000_000):
+    """One step of SpectralPipeline.run_device as .npy files in out_dir: what it returns to its caller (eigenvalues
+    [B, K], eigenvectors [B, K, N] float32; the eigensolver's info [B, 4] -- Lanczos steps, converged flag, ... -- as
+    float64) and the K features [B, N, d] it computed on the way. The features are kept for a fixed seeded sample of `feature_images` images (all
+    of them are 400 MB at the default step); the other arrays are sampled the same way only where all images would not
+    fit in `budget` bytes. image_index.npy / features_image_index.npy give the image of each row."""
+    import numpy as np
+    import torch
+    B = evals.shape[0]
+    order = np.random.default_rng(0).permutation(B)
+    feat_bytes = feats[0].numel() * 4 + 8
+    n_feat = min(B, feature_images, budget // 2 // feat_bytes)
+    eig_bytes = (evals[0].numel() + evecs[0].numel()) * 4 + (info[0].numel() + 1) * 8
+    n_eig = min(B, (budget - n_feat * feat_bytes) // eig_bytes)
+    eig_rows = np.arange(B) if n_eig == B else np.sort(order[:n_eig])
+    feat_rows = np.sort(order[:n_feat])
+
+    def rows(t, r, dtype):
+        return t[torch.from_numpy(r).to(t.device)].cpu().numpy().astype(dtype)
+    arrays = {"eigenvalues": rows(evals, eig_rows, np.float32), "eigenvectors": rows(evecs, eig_rows, np.float32),
+              "lanczos_info": rows(info, eig_rows, np.float64), "image_index": eig_rows.astype(np.float64),
+              "features": rows(feats, feat_rows, np.float32), "features_image_index": feat_rows.astype(np.float64)}
+    assert sum(a.nbytes for a in arrays.values()) <= budget
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_c2(ctx: Ctx):
     args, torch, dev = ctx.args, ctx.torch, ctx.dev
     import numpy as np
@@ -534,6 +570,9 @@ def run_c2(ctx: Ctx):
     def step_dev():
         last["out"] = pipe.run_device(dev_imgs)
     ms, launches = ctx.timed(step_dev, steps, W)
+    if args.dump_outputs and ctx.rank == 0:
+        # now: the end-to-end pass below reuses the feature buffer of this step
+        dump_outputs(args.dump_outputs, *last["out"], pipe._bufs["feats"])
     value = ctx.world * B * steps / (ms * 1e-3)
     info = last["out"][2]
     conv = int(info[:, 1].sum().item())

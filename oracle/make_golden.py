@@ -2,6 +2,7 @@
 oracle/ref_shim.py) on small seeded inputs. Run in the dev container only:
 
     python -m oracle.make_golden
+    python -m oracle.make_golden --reference-calls    # only the ref_*.npz fixtures
 
 Each fixture stores the inputs (features, optional JPEG bytes + the low-res image the reference derived from it)
 and the tensors the reference saved. tests/test_cpu_oracle.py checks the oracle restatement against them;
@@ -101,12 +102,58 @@ def make_segmentation_golden():
         print(name, "labels:", np.unique(multi), "single on:", int((single > 0).sum()))
 
 
+def make_reference_call_golden():
+    """ref_*.npz: inputs and outputs of three direct calls of the reference's functions (its _extract_eig, its
+    utils.knn_affinity, its two segmentation workers and utils.get_border_fraction). tests/test_cpu_oracle.py checks the
+    oracle against these recorded outputs, so the checks run wherever the tests run."""
+    from PIL import Image
+    ref = ref_shim.load_reference()
+    # _extract_eig with the default flags
+    feats = synth.structured_features(150, 64, 6, 42)
+    fd = {"k": feats[None], "indices": torch.tensor(0), "file": "x.jpg", "id": "x", "model_name": "dino_vits16",
+          "patch_size": 16, "shape": (1, 3, 160, 240)}
+    with tempfile.TemporaryDirectory() as td:
+        out = ref_shim.run_reference_extract_eig(fd, td, K=6)
+    np.savez_compressed(GOLDEN / "ref_extract_eig_150_k6.npz", feats=feats.numpy(), K=6,
+                        eigenvalues=np.asarray(out["eigenvalues"]), eigenvectors=out["eigenvectors"].numpy())
+    # utils.knn_affinity on a 12 x 15 low-resolution image
+    img = synth.blobs_image(12 * 16, 15 * 16, 7).numpy()
+    lr = np.array(Image.fromarray(img).resize((15, 12), Image.BILINEAR)) / 255.0
+    W = ref_shim.reference_knn_affinity(lr).tocoo()
+    np.savez_compressed(GOLDEN / "ref_knn_affinity_12x15.npz", image_lr=lr, shape=np.array(W.shape),
+                        row=W.row.astype(np.int32), col=W.col.astype(np.int32), data=W.data)
+    # the single- and multi-region workers on a 7 x 11 patch grid, and the border fractions of the multi-region PNG
+    vals, vecs, feats, band = planted_eigs(7, 11, 4, 17)
+    kw = dict(adaptive=True, non_adaptive_num_segments=4, infer_bg_index=True, kmeans_baseline=False, num_eigenvectors=3)
+    with tempfile.TemporaryDirectory() as td:
+        fdir, edir, o1, o2 = (Path(td) / n for n in ("f", "e", "s", "m"))
+        for d in (fdir, edir, o1, o2):
+            d.mkdir()
+        fd = {"k": feats[None], "indices": torch.tensor(0), "file": "x.jpg", "id": "x", "model_name": "dino_vits16",
+              "patch_size": 16, "shape": (1, 3, 7 * 16 + 3, 11 * 16)}
+        torch.save(fd, fdir / "x.pth")
+        torch.save({"eigenvalues": vals, "eigenvectors": vecs}, edir / "x.pth")
+        inp = ref.utils.get_paired_input_files(str(fdir), str(edir))[0]
+        ref._extract_single_region_segmentations(inp, threshold=0.0, output_dir=str(o1))
+        np.random.seed(7)        # the reference's KMeans is unseeded: k-means++ draws from numpy's global RNG
+        ref._extract_multi_region_segmentations(inp, output_dir=str(o2), **kw)
+        single, multi = np.array(Image.open(o1 / "x.png")), np.array(Image.open(o2 / "x.png"))
+    border_idx, border_frac = ref.utils.get_border_fraction(multi)
+    np.savez_compressed(GOLDEN / "ref_segment_7x11.npz", eigenvalues=vals.numpy(), eigenvectors=vecs.numpy(),
+                        feats=feats.numpy(), grid=np.array([7, 11]), kwargs=np.array(repr(kw)), threshold=0.0, rng_seed=7,
+                        single=single, multi=multi, border_indices=np.asarray(border_idx),
+                        border_fractions=np.asarray(border_frac))
+    print("reference calls recorded: lambda", np.asarray(out["eigenvalues"]), "labels", np.unique(multi))
+
 
 def main():
     assert ref_shim.available(), "reference sources not present"
     GOLDEN.mkdir(parents=True, exist_ok=True)
     from PIL import Image
     import sys as _sys
+    if "--reference-calls" in _sys.argv:
+        make_reference_call_golden()
+        return
     regenerate_all = "--all" in _sys.argv
     for name, (Hp, Wp), d, K, rank, seed, kw in CASES:
         if not regenerate_all and name not in ONLY_NEW and (GOLDEN / f"{name}.npz").is_file():

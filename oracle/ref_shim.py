@@ -1,8 +1,7 @@
 """ORACLE (test infrastructure, not product): run the reference's *own* ``_extract_eig`` in this container.
 
-/root/reference is read-only and exists only in the dev container (never on the GPU box), so nothing in the
-``-m gpu`` tests, smoke() or bench.py imports this file; it is used by oracle/make_golden.py to produce the
-committed fixtures under tests/golden/ and by tests/test_oracle_golden.py (skipped when the reference is absent).
+The reference's sources are only needed where the fixtures are generated, so no test, smoke() or bench.py imports
+this file; oracle/make_golden.py uses it to record the fixtures under tests/golden/, which the tests compare with.
 
 The reference's module imports packages that are not installed here (fire, accelerate, skimage, pymatting); they
 are replaced by inert stubs *before* ``import extract``:

@@ -31,6 +31,7 @@ def test_library_exports_every_declared_symbol():
 def test_bad_arguments_are_rejected_before_any_device_work():
     _lib = load_pkg("_lib")
     lib = _lib.load()
+    launches_before = lib.dss_kernel_launch_count()     # the counter is per process: GPU tests may have run before
     assert lib.dss_affinity(None, 1, 10, 8, 3, None, 0.0, None, 12, None, None, 0, None) == -1
     assert b"null" in lib.dss_last_error()
     buf = torch.zeros(1 << 16, dtype=torch.uint8)
@@ -51,7 +52,7 @@ def test_bad_arguments_are_rejected_before_any_device_work():
     assert lib.dss_vit_forward_k(h, p, 1, 224, 224, -1, p, p, 1 << 15, None) == -1          # weights not loaded
     lib.dss_vit_destroy(h)
     assert lib.dss_affinity_workspace_bytes(2, 900, 384) >= 2 * 900 * 384 * 4
-    assert lib.dss_kernel_launch_count() == 0                                               # nothing was launched
+    assert lib.dss_kernel_launch_count() == launches_before                                 # nothing was launched
 
 
 @pytest.mark.parametrize("name,Hp,Wp", [("dino_vits16", 30, 30), ("dino_vits16", 23, 31), ("dino_vits16", 14, 14),

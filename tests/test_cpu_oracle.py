@@ -1,6 +1,6 @@
 """CPU suite: the oracle (oracle/eigs_ref.py, oracle/dino_vit.py) is pinned against
   * the committed golden fixtures produced by the reference's own _extract_eig (tests/golden/, oracle/make_golden.py),
-  * the reference itself when /root/reference is present (dev container only),
+  * recorded outputs of direct calls of the reference's functions (tests/golden/ref_*.npz, same generator),
   * analytic known-answer cases and an independent ViT implementation (transformers.ViTModel)."""
 import ast
 import io
@@ -11,10 +11,11 @@ import pytest
 import torch
 
 from conftest import ROOT, load_pkg
-from oracle import dino_vit, eigs_ref, ref_shim
+from oracle import dino_vit, eigs_ref
 
-GOLDEN = sorted((ROOT / "tests" / "golden").glob("lap_*.npz"))
-SEG_GOLDEN = sorted((ROOT / "tests" / "golden").glob("seg_*.npz"))
+GOLDEN_DIR = ROOT / "tests" / "golden"
+GOLDEN = sorted(GOLDEN_DIR.glob("lap_*.npz"))
+SEG_GOLDEN = sorted(GOLDEN_DIR.glob("seg_*.npz"))
 torch.set_grad_enabled(False)
 
 
@@ -65,26 +66,22 @@ def test_oracle_reproduces_reference_golden(path):
     assert np.all(_aligned_err(vec.numpy(), z["eigenvectors"]) <= gap_tolerance(feats, int(z["K"]), kw))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference sources only exist in the dev container")
-def test_oracle_matches_live_reference(tmp_path):
-    synth = load_pkg("synth")
-    feats = synth.structured_features(150, 64, 6, 42)
-    fd = {"k": feats[None], "indices": torch.tensor(0), "file": "x.jpg", "id": "x", "model_name": "dino_vits16",
-          "patch_size": 16, "shape": (1, 3, 160, 240)}
-    out = ref_shim.run_reference_extract_eig(fd, tmp_path, K=6)
-    ev, vec = eigs_ref.extract_eig(feats, 6, rng_seed=1)
-    assert np.abs(ev.numpy() - np.asarray(out["eigenvalues"])).max() <= 2e-6
-    assert _aligned_err(vec.numpy(), out["eigenvectors"].numpy()).max() <= 2e-5
-    assert out["eigenvectors"].dtype == torch.float32 and tuple(out["eigenvectors"].shape) == (6, 150)
+def test_oracle_matches_live_reference():
+    """Against what the reference's _extract_eig returned for these features (tests/golden/ref_extract_eig_150_k6.npz,
+    recorded by ``python -m oracle.make_golden --reference-calls``)."""
+    z = np.load(GOLDEN_DIR / "ref_extract_eig_150_k6.npz")
+    ev, vec = eigs_ref.extract_eig(torch.from_numpy(z["feats"]), int(z["K"]), rng_seed=1)
+    assert np.abs(ev.numpy() - z["eigenvalues"]).max() <= 2e-6
+    assert _aligned_err(vec.numpy(), z["eigenvectors"]).max() <= 2e-5
+    assert z["eigenvectors"].dtype == np.float32 and z["eigenvectors"].shape == (6, 150)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference sources only exist in the dev container")
 def test_knn_affinity_restatement_matches_reference_function():
-    synth = load_pkg("synth")
-    img = synth.blobs_image(12 * 16, 15 * 16, 7).numpy()
-    from PIL import Image
-    lr = np.array(Image.fromarray(img).resize((15, 12), Image.BILINEAR)) / 255.0
-    W_ref = ref_shim.reference_knn_affinity(lr).toarray()
+    """Against the matrix the reference's utils.knn_affinity returned for this image (ref_knn_affinity_12x15.npz)."""
+    from scipy.sparse import coo_matrix
+    z = np.load(GOLDEN_DIR / "ref_knn_affinity_12x15.npz")
+    lr = z["image_lr"]
+    W_ref = coo_matrix((z["data"], (z["row"], z["col"])), shape=tuple(z["shape"])).toarray()
     W = eigs_ref.knn_affinity(lr).toarray()
     assert np.array_equal(W, W_ref)
     assert np.array_equal(W, W.T) and set(np.unique(W)) <= {0.0, 1.0, 2.0, 3.0, 4.0} and np.all(np.diag(W) == 4)
@@ -200,32 +197,19 @@ def test_segmentation_oracle_reproduces_reference_golden(path):
     assert segment_ref.same_partition(multi, z["band"])          # and it is the planted partition
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference sources only exist in the dev container")
-def test_segmentation_oracle_matches_live_reference(tmp_path):
-    from PIL import Image
-    from oracle import make_golden, segment_ref
-    ref = ref_shim.load_reference()
-    vals, vecs, feats, band = make_golden.planted_eigs(7, 11, 4, 17)
-    fdir, edir, o1, o2 = (tmp_path / n for n in ("f", "e", "s", "m"))
-    for d in (fdir, edir, o1, o2):
-        d.mkdir()
-    fd = {"k": feats[None], "indices": torch.tensor(0), "file": "x.jpg", "id": "x", "model_name": "dino_vits16",
-          "patch_size": 16, "shape": (1, 3, 7 * 16 + 3, 11 * 16)}
-    torch.save(fd, fdir / "x.pth")
-    torch.save({"eigenvalues": vals, "eigenvectors": vecs}, edir / "x.pth")
-    inp = ref.utils.get_paired_input_files(str(fdir), str(edir))[0]
-    ref._extract_single_region_segmentations(inp, threshold=0.0, output_dir=str(o1))
-    kw = dict(adaptive=True, non_adaptive_num_segments=4, infer_bg_index=True, kmeans_baseline=False, num_eigenvectors=3)
-    np.random.seed(7)
-    ref._extract_multi_region_segmentations(inp, output_dir=str(o2), **kw)
-    assert np.array_equal(np.array(Image.open(o1 / "x.png")), segment_ref.single_region(vecs.numpy(), 7, 11, 0.0))
-    np.random.seed(7)
-    assert np.array_equal(np.array(Image.open(o2 / "x.png")),
-                          segment_ref.multi_region(vals.numpy(), vecs.numpy(), feats.numpy(), 7, 11, **kw))
-    seg = np.array(Image.open(o2 / "x.png"))
-    i1, c1 = segment_ref.get_border_fraction(seg)
-    i2, c2 = ref.utils.get_border_fraction(seg)
-    assert np.array_equal(i1, i2) and np.array_equal(c1, c2)
+def test_segmentation_oracle_matches_live_reference():
+    """Against the PNGs the reference's two segmentation workers wrote for these eigenvectors and the border fractions
+    its utils.get_border_fraction returned for the multi-region one (ref_segment_7x11.npz)."""
+    from oracle import segment_ref
+    z = np.load(GOLDEN_DIR / "ref_segment_7x11.npz")
+    kw = ast.literal_eval(str(z["kwargs"]))
+    Hp, Wp = (int(v) for v in z["grid"])
+    vals, vecs, feats = z["eigenvalues"], z["eigenvectors"], z["feats"]
+    assert np.array_equal(z["single"], segment_ref.single_region(vecs, Hp, Wp, float(z["threshold"])))
+    np.random.seed(int(z["rng_seed"]))           # the RNG state the reference's K-means started from
+    assert np.array_equal(z["multi"], segment_ref.multi_region(vals, vecs, feats, Hp, Wp, **kw))
+    i1, c1 = segment_ref.get_border_fraction(z["multi"])
+    assert np.array_equal(i1, z["border_indices"]) and np.array_equal(c1, z["border_fractions"])
 
 
 def test_rw_affinity_restatement_properties():
