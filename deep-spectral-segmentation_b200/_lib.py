@@ -55,7 +55,6 @@ PROTOTYPES = {
                                 c_int, c_void_p]),
     "dss_op_gemm_f16_simt": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
                                      c_int, c_int, c_void_p]),
-    "dss_debug_gemm_cfg": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "dss_op_gemm_ln_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float,
                                    c_int, c_void_p]),
     "dss_op_layernorm_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_void_p]),

@@ -3,6 +3,7 @@
 #include <stdio.h>
 
 #include <atomic>
+#include <map>
 #include <mutex>
 #include <utility>
 #include <vector>
@@ -30,6 +31,20 @@ int device_sm_count() {
   if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return -1;
   cached[dev] = n;
   return n;
+}
+
+cudaError_t allow_dynamic_smem(const void* kernel, int bytes) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, int> allowed;   // (kernel, device) -> bytes
+  std::lock_guard<std::mutex> lk(mu);
+  int& have = allowed[{kernel, dev}];
+  if (bytes <= have) return cudaSuccess;
+  e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e == cudaSuccess) have = bytes;
+  return e;
 }
 
 // ---- launch counter + optional per-class event timing

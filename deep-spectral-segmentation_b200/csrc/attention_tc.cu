@@ -24,10 +24,6 @@
 // group's MUFU-bound exp phase overlaps the other's TMEM loads / maxima / fences. The kernel is bound by the MUFU pipe
 // (128 x 128 exp2 per tile at 16 per clock per SM), not by the tensor pipe.
 #include <math.h>
-#include <stdio.h>
-#include <stdlib.h>
-
-#include <type_traits>
 
 #include "common.cuh"
 
@@ -76,23 +72,11 @@ constexpr int FA_SMEM = FA_TILE * (4 + 2 * FA_KV_STAGES + 2);
 constexpr int FA_TMEM_COLS = 512;
 constexpr int FA_S_COL = 0, FA_O_COL = 256, FA_P_COL = 384;   // S_A, S_B at 0 / 128; O_A, O_B at 256 / 320; P_A, P_B at 384 / 448
 constexpr float FA_RESCALE_LOG2 = 8.0f;       // raise the reference maximum only when exceeded by more than 2^8
-#ifdef DSS_ATTN_ABLATION
-__device__ long long* g_attn_trace = nullptr;   // tuning only: per-phase clock64 stamps of CTA 0
-#define FA_TRACE(slot) do { if (trace) trace[(slot)] = clock64(); } while (0)
-#else
-#define FA_TRACE(slot) do { } while (0)
-#endif
 constexpr int FA_NBARS = 8 + 2 * FA_KV_STAGES + 10;
 
-// ABL: timing-ablation bits (tuning only; any non-zero value computes garbage): 1 no exp2, 2 no P stores / fence,
-// 4 no row maximum, 8 no P V MMAs, 16 no score MMAs, 32 no row sum
-template <int ABL>
 __global__ void __launch_bounds__(FA_THREADS, 1)
 attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmO, int T, int heads,
-                         int nq2, int total_items, int flags) {
-  // flags (tuning switches, both on by default): 1 = rotate the query-pair index over the items, 2 = take the exponentials
-  // of tiles j > 0 against the reference maximum of the earlier tiles (no separate row-maximum pass)
-  const bool f_rotate = flags & 1, f_lazy = flags & 2;
+                         int nq2, int total_items) {
   extern __shared__ __align__(1024) uint8_t fa_smem[];
   __shared__ __align__(8) uint64_t bars[FA_NBARS];
   __shared__ uint32_t tmem_ptr_s;
@@ -111,9 +95,6 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
   auto s_free = [&](int g) { return bar0 + 8u * (16 + 2 * FA_KV_STAGES + g); };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#ifdef DSS_ATTN_ABLATION
-  long long* trace = (blockIdx.x == 0 && lane == 0 && (warp == 1 || warp == 2 || warp >= 4)) ? g_attn_trace : nullptr;
-#endif
   const int d = heads * FA_D;
   const int nt = (T + FA_BN - 1) / FA_BN;
   const int kc_last = (T - (nt - 1) * FA_BN + 15) & ~15;   // key columns of the last tile that are worth computing
@@ -162,7 +143,7 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
       // with the plain w % nq2 a CTA (w = blockIdx + k * 148, 148 % 4 == 0) would get the SAME pair index in every item,
       // and the CTAs that only ever see the light last pair (a 5-row tail tile at T = 901) idle at the end of the
       // kernel while the others are still on full pairs (ncu: 8.5 % of the stall samples on EXIT)
-      const int bh = w / nq2, qp = f_rotate ? (w % nq2 + bh) % nq2 : w % nq2;
+      const int bh = w / nq2, qp = (w % nq2 + bh) % nq2;
       const int h = bh % heads, row0 = (bh / heads) * T;   // first row of this image in the [B*T, 3d] matrix
       const int qb = qi & 1;
       const uint32_t qph = (qi >> 1) & 1;
@@ -214,7 +195,7 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
       if (elect_one()) {
 #pragma unroll
         for (int k = 0; k < FA_D / 16; ++k)   // +32 B per 16-wide K step = +2 in the descriptor's address field
-          if (!(ABL & 16)) umma_f16_ss(s_acc, qdesc + 2u * k, kdesc + 2u * k, idesc, k != 0 ? 1u : 0u);
+          umma_f16_ss(s_acc, qdesc + 2u * k, kdesc + 2u * k, idesc, k != 0 ? 1u : 0u);
         umma_commit(s_full(g));
         if (sj == nt - 1) umma_commit(q_empty(g, sq & 1));   // last score tile of the item: Q_g may be replaced
       }
@@ -227,27 +208,23 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
     for (int n = 0; n < m_total; ++n) {
       if (n + 1 < m_total) {   // S_g(n+1) as soon as the softmax warps hold S_g(n) in registers
         mbar_wait(s_free(g), n & 1);
-        FA_TRACE(8192 + g * 2048 + (n < 500 ? n : 500) * 4 + 0);
         issue_s();
-        FA_TRACE(8192 + g * 2048 + (n < 500 ? n : 500) * 4 + 1);
       }
       // O_g (+)= P_g V_j once the softmax warps have published P_g(n) (and rescaled O_g if they had to)
       mbar_wait(p_full(g), n & 1);
       tc_fence_after();
-      FA_TRACE(8192 + g * 2048 + (n < 500 ? n : 500) * 4 + 2);
       const int ksteps = (pj == nt - 1 ? kc_last : FA_BN) >> 4;
       const uint64_t vdesc = umma_desc_sw128(uV + ps * FA_TILE);   // +16 key rows = +2048 B = +128
       const bool first = pj == 0;   // first key tile of the item: overwrite
       if (elect_one()) {
 #pragma unroll
         for (int k = 0; k < FA_BN / 16; ++k)
-          if (k < ksteps && !(ABL & 8))
+          if (k < ksteps)
             umma_f16_ts(o_acc, p_tm + 8u * k, vdesc + 128u * k, idesc_pv, (k != 0 || !first) ? 1u : 0u);
         umma_commit(o_full(g));
         umma_commit(kv_empty(ps));   // this query tile is done with K_j / V_j (the ring slot needs both tiles' commits)
       }
       __syncwarp();
-      FA_TRACE(8192 + g * 2048 + (n < 500 ? n : 500) * 4 + 3);
       if (++pj == nt) pj = 0;
       if (++ps == FA_KV_STAGES) ps = 0;
     }
@@ -268,10 +245,10 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
       // with the plain w % nq2 a CTA (w = blockIdx + k * 148, 148 % 4 == 0) would get the SAME pair index in every item,
       // and the CTAs that only ever see the light last pair (a 5-row tail tile at T = 901) idle at the end of the
       // kernel while the others are still on full pairs (ncu: 8.5 % of the stall samples on EXIT)
-      const int bh = w / nq2, qp = f_rotate ? (w % nq2 + bh) % nq2 : w % nq2;
+      const int bh = w / nq2, qp = (w % nq2 + bh) % nq2;
       const int h = bh % heads;
       const int q0 = (2 * qp + g) * FA_BM;
-      const bool dead = q0 >= T || ((ABL & 64) && g == 1);   // odd number of query tiles: nothing to do for B in the last pair
+      const bool dead = q0 >= T;   // odd number of query tiles: nothing to do for B in the last pair
       // a warp whose 32 query rows all lie beyond T (T = 901: three of the four warps of the 8th tile, which has 5 live
       // rows) only keeps the barrier protocol going: its exponentials would occupy the MUFU unit -- the busiest unit of
       // the kernel -- for rows the output tensor map clips anyway
@@ -283,8 +260,6 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
         if (j == 0 && g == 1) { __syncwarp(); asm volatile("bar.sync 3, 256;" ::: "memory"); }
         mbar_wait(s_full(g), m & 1);
         tc_fence_after();
-        [[maybe_unused]] const int tb = (warp - 4) * 1024 + (m < 120 ? m : 120) * 8;   // trace slot (ablation builds)
-        FA_TRACE(tb + 0);
         if (!wdead) {
           // one key tile, in four chunks of 32 key columns; only the last tile of a row of tiles can be short
           // (kc < 128 columns computed, nvalid <= kc of them real keys)
@@ -306,7 +281,7 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
             if (track_max) {
 #pragma unroll
               for (int i = c * 32; i < c * 32 + 32; ++i)
-                if (!(ABL & 4)) mxc[i & 3] = fmaxf(mxc[i & 3], __uint_as_float(v[i]));
+                mxc[i & 3] = fmaxf(mxc[i & 3], __uint_as_float(v[i]));
             }
             const uint64_t sc2 = pack_f32x2(sc, sc), nmsc2 = pack_f32x2(-msc, -msc);
             uint32_t pk[16];
@@ -315,66 +290,38 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
               const int i = c * 32 + e;
               float x0, x1;
               unpack_f32x2(fma_f32x2(pack_f32x2(__uint_as_float(v[i]), __uint_as_float(v[i + 1])), sc2, nmsc2), x0, x1);
-              constexpr int npoly = (ABL & 1024) ? 0 : ((ABL >> 8) & 3) ? ((ABL >> 8) & 3) : FA_POLY_OF_4;
               float p0, p1;
-              if (((e >> 1) & 3) < npoly) {
+              if (((e >> 1) & 3) < FA_POLY_OF_4) {
                 ex2_poly_x2(x0, x1, p0, p1);
               } else {
-                p0 = (ABL & 1) ? x0 : ex2_approx(x0);
-                p1 = (ABL & 1) ? x1 : ex2_approx(x1);
+                p0 = ex2_approx(x0);
+                p1 = ex2_approx(x1);
               }
-              if (!(ABL & 32)) rs2[(e >> 1) & 1] = add_f32x2(rs2[(e >> 1) & 1], pack_f32x2(p0, p1));
+              rs2[(e >> 1) & 1] = add_f32x2(rs2[(e >> 1) & 1], pack_f32x2(p0, p1));
               pk[e >> 1] = pack_half2(p0, p1);
             }
-            if (!(ABL & 2)) tmem_st_32x16(p_col + c * 16, pk);
-            else rs2[0] += pk[0] ^ pk[5] ^ pk[10] ^ pk[15];   // keep the values alive
+            tmem_st_32x16(p_col + c * 16, pk);
           };
 #pragma unroll
           for (int c = 0; c < 4; ++c)
             if (c * 32 < kc) tmem_ld_32x32(s_col + c * 32, *reinterpret_cast<uint32_t (*)[32]>(&v[c * 32]));
           tmem_ld_wait();
-          FA_TRACE(tb + 1);
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(s_free(g));   // S_g is in registers: the next score tile may overwrite it
-          if (j == 0 || !f_lazy) {
-            // ---- the row maximum first (always for the first key tile of an item: there is no reference yet)
+          if (j == 0) {
+            // ---- first key tile of an item: there is no reference yet, so the row maximum comes first
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
               if (c * 32 < kc) {
 #pragma unroll
                 for (int i = c * 32; i < c * 32 + 32; ++i) {
                   if (tail && i >= nvalid) v[i] = 0xff800000u;
-                  if (!(ABL & 4)) mxc[i & 3] = fmaxf(mxc[i & 3], __uint_as_float(v[i]));
+                  mxc[i & 3] = fmaxf(mxc[i & 3], __uint_as_float(v[i]));
                 }
               }
             }
-            const float mx = fmaxf(fmaxf(mxc[0], mxc[1]), fmaxf(mxc[2], mxc[3]));
-            FA_TRACE(tb + 2);
-            if (j > 0) {
-              // P_g is single buffered and O_g accumulates in place: P_g V_{j-1} must be complete (issued long ago)
-              mbar_wait(o_full(g), (m - 1) & 1);
-              tc_fence_after();
-              const bool raise = (mx - m_ref) * sc > FA_RESCALE_LOG2;
-              if (__any_sync(0xffffffffu, raise)) {   // rare: rescale this warp's rows of O_g in TMEM
-                const float f = raise ? ex2_approx((m_ref - mx) * sc) : 1.0f;
-                uint32_t t[32];
-#pragma unroll
-                for (int c = 0; c < 2; ++c) {
-                  tmem_ld_32x32(o_col + c * 32, t);
-                  tmem_ld_wait();
-#pragma unroll
-                  for (int i = 0; i < 32; ++i) t[i] = __float_as_uint(__uint_as_float(t[i]) * f);
-                  tmem_st_32x32(o_col + c * 32, t);
-                }
-                tmem_st_wait();
-                l_run *= f;
-                if (raise) m_ref = mx;
-              }
-            } else {
-              m_ref = mx;
-            }
-            FA_TRACE(tb + 3);
+            m_ref = fmaxf(fmaxf(mxc[0], mxc[1]), fmaxf(mxc[2], mxc[3]));
             const float msc = m_ref * sc;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
@@ -382,10 +329,10 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
                 chunk(c, msc, false);
                 // release tile B's first key tile when tile A is half way through its first exponentials: the two
                 // groups then stay about half a period apart (one in its MUFU phase, the other loading / reducing)
-                if (c == 1 && j == 0 && g == 0) { __syncwarp(); asm volatile("bar.arrive 3, 256;" ::: "memory"); }
+                if (c == 1 && g == 0) { __syncwarp(); asm volatile("bar.arrive 3, 256;" ::: "memory"); }
               }
             }
-            if (kc <= 32 && j == 0 && g == 0) { __syncwarp(); asm volatile("bar.arrive 3, 256;" ::: "memory"); }   // (short first tile)
+            if (kc <= 32 && g == 0) { __syncwarp(); asm volatile("bar.arrive 3, 256;" ::: "memory"); }   // (short first tile)
           } else {
             // ---- later key tiles: exponentials are taken relative to the reference maximum of the EARLIER tiles right
             // away (softmax is shift invariant; fp16 P and the fp32 sums have 2^8 of headroom) with the row maximum
@@ -393,12 +340,10 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
             // 2^8 is the reference raised and the tile redone (rare).
             mbar_wait(o_full(g), (m - 1) & 1);   // P_g is single buffered: P_g V_{j-1} must be complete
             tc_fence_after();
-            FA_TRACE(tb + 2);
             float msc = m_ref * sc;
 #pragma unroll
             for (int c = 0; c < 4; ++c)
               if (c * 32 < kc) chunk(c, msc, true);
-            FA_TRACE(tb + 3);
             const float mx = fmaxf(fmaxf(mxc[0], mxc[1]), fmaxf(mxc[2], mxc[3]));
             const bool raise = (mx - m_ref) * sc > FA_RESCALE_LOG2;
             if (__any_sync(0xffffffffu, raise)) {   // rare: rescale this warp's rows of O_g in TMEM, redo the tile
@@ -426,13 +371,11 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
           float rs, rs_hi;
           unpack_f32x2(add_f32x2(rs2[0], rs2[1]), rs, rs_hi);
           rs += rs_hi;
-          FA_TRACE(tb + 4);
           l_run += rs;
           tmem_st_wait();
           tc_fence_before();          // order this thread's TMEM accesses before the MMA that accumulates into O_g
           __syncwarp();
           if (lane == 0) mbar_arrive(p_full(g));
-          FA_TRACE(tb + 5);
         } else {
           // nothing to compute, but keep the protocol: P_g(m) may only be announced once P_g V(m-1) has been issued
           // (the MMA warp probes p_full by parity and must never be lapped by two phases)
@@ -496,55 +439,18 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
 
 int launch_attention_tc(const void* qkv, void* out, int B, int T, int heads, cudaStream_t st) {
   DSS_REQUIRE(B > 0 && T > 0 && heads > 0, "attention: empty problem");
-  static int flags = 3;
-  static int abl = -1;
-  if (abl < 0) {
-    if (const char* e = getenv("DSS_ATTN_FLAGS")) flags = atoi(e);   // tuning: bit 0 item rotation, bit 1 lazy reference
-    const char* e = getenv("DSS_ATTN_ABL");   // tuning only
-    abl = e ? atoi(e) : 0;
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(attention_tcgen05_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
-#ifdef DSS_ATTN_ABLATION
-#define DSS_ABL_ATTR(n) DSS_CHECK_CUDA(cudaFuncSetAttribute(attention_tcgen05_kernel<n>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
-    DSS_ABL_ATTR(1) DSS_ABL_ATTR(2) DSS_ABL_ATTR(4) DSS_ABL_ATTR(8) DSS_ABL_ATTR(16) DSS_ABL_ATTR(32) DSS_ABL_ATTR(3) DSS_ABL_ATTR(7) DSS_ABL_ATTR(39) DSS_ABL_ATTR(24) DSS_ABL_ATTR(63) DSS_ABL_ATTR(64) DSS_ABL_ATTR(65) DSS_ABL_ATTR(127) DSS_ABL_ATTR(88) DSS_ABL_ATTR(256) DSS_ABL_ATTR(512) DSS_ABL_ATTR(768) DSS_ABL_ATTR(1024)
-#endif
-  }
+  DSS_CHECK_CUDA(allow_dynamic_smem(attention_tcgen05_kernel, FA_SMEM));
   CUtensorMap tm, tmO;
   int rc = make_tmap_f16(&tm, qkv, B * T, 3 * heads * FA_D, FA_BM);
   if (rc) return rc;
   if ((rc = make_tmap_out3d_f16(&tmO, out, B, T, heads * FA_D))) return rc;
-  static int sm_count = 0;
-  if (!sm_count) {
-    int dev = 0;
-    DSS_CHECK_CUDA(cudaGetDevice(&dev));
-    DSS_CHECK_CUDA(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev));
-  }
+  int sms = device_sm_count();
+  if (sms <= 0) sms = 148;
   const int nq2 = cdiv(cdiv(T, FA_BM), 2);   // pairs of 128-query tiles per (image, head)
   const int total = B * heads * nq2;
-  const int grid = total < sm_count ? total : sm_count;   // persistent: one CTA per SM
+  const int grid = total < sms ? total : sms;   // persistent: one CTA per SM
   LaunchScope scope(st, KC_ATTENTION);
-#ifdef DSS_ATTN_ABLATION
-  static long long* trace_dev = nullptr;
-  const char* trace_path = getenv("DSS_ATTN_TRACE");
-  if (trace_path && !trace_dev) {
-    DSS_CHECK_CUDA(cudaMalloc(&trace_dev, 16384 * sizeof(long long)));
-    DSS_CHECK_CUDA(cudaMemset(trace_dev, 0, 16384 * sizeof(long long)));
-    DSS_CHECK_CUDA(cudaMemcpyToSymbol(g_attn_trace, &trace_dev, sizeof(trace_dev)));
-  }
-#define DSS_ABL_CASE(n) case n: attention_tcgen05_kernel<n><<<grid, FA_THREADS, FA_SMEM, st>>>(tm, tmO, T, heads, nq2, total, flags); break;
-  switch (abl) {
-    DSS_ABL_CASE(1) DSS_ABL_CASE(2) DSS_ABL_CASE(4) DSS_ABL_CASE(8) DSS_ABL_CASE(16) DSS_ABL_CASE(32) DSS_ABL_CASE(3) DSS_ABL_CASE(7) DSS_ABL_CASE(39) DSS_ABL_CASE(24) DSS_ABL_CASE(63) DSS_ABL_CASE(64) DSS_ABL_CASE(65) DSS_ABL_CASE(127) DSS_ABL_CASE(88) DSS_ABL_CASE(256) DSS_ABL_CASE(512) DSS_ABL_CASE(768) DSS_ABL_CASE(1024)
-    default: attention_tcgen05_kernel<0><<<grid, FA_THREADS, FA_SMEM, st>>>(tm, tmO, T, heads, nq2, total, flags);
-  }
-  if (trace_path) {
-    static long long host[16384];
-    DSS_CHECK_CUDA(cudaStreamSynchronize(st));
-    DSS_CHECK_CUDA(cudaMemcpy(host, trace_dev, sizeof(host), cudaMemcpyDeviceToHost));
-    FILE* f = fopen(trace_path, "wb");
-    if (f) { fwrite(host, sizeof(host), 1, f); fclose(f); }
-  }
-#else
-  attention_tcgen05_kernel<0><<<grid, FA_THREADS, FA_SMEM, st>>>(tm, tmO, T, heads, nq2, total, flags);
-#endif
+  attention_tcgen05_kernel<<<grid, FA_THREADS, FA_SMEM, st>>>(tm, tmO, T, heads, nq2, total);
   DSS_CHECK_CUDA(cudaGetLastError());
   return DSS_OK;
 }

@@ -465,4 +465,12 @@ __device__ __forceinline__ float warp_max(float v) {
 
 #endif  // __CUDACC__
 
+// Lets `kernel` be launched with up to `bytes` of dynamic shared memory on the current device. The limit is a property
+// of the kernel in that device's context, so it is set once per kernel and device (again only to raise it); thread-safe.
+cudaError_t allow_dynamic_smem(const void* kernel, int bytes);
+template <class Kernel>
+inline cudaError_t allow_dynamic_smem(Kernel* kernel, int bytes) {
+  return allow_dynamic_smem(reinterpret_cast<const void*>(kernel), bytes);
+}
+
 }  // namespace dss

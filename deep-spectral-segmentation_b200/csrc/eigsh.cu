@@ -8,7 +8,7 @@
 //
 // One persistent CTA per image: the whole iteration (mat-vec, re-orthogonalisation, Ritz extraction, convergence
 // test) runs inside one kernel with block-level barriers only; images are independent, so a batch fills the GPU
-// with one CTA (or more) per SM and nothing ever synchronises across CTAs. The mat-vec is the only HBM stream of the
+// with one CTA per SM and nothing ever synchronises across CTAs. The mat-vec is the only HBM stream of the
 // kernel and W is symmetric, so only its UPPER TRIANGLE is read: row r contributes W[r, c >= r] x[c] to y[r] (warp
 // reduction) and W[r, c > r] x[r] to y[c] (per-lane column accumulators in registers, combined across warps through
 // shared memory once per mat-vec) -- 2 N^2 bytes per step instead of 4 N^2. The degree D = W 1 comes from the
@@ -16,7 +16,6 @@
 // The Lanczos basis lives in a per-CTA global scratch (L2), the working vectors in shared memory. Ritz values of the tridiagonal matrix come from a 32-way
 // Sturm multisection in fp64 (one warp per eigenvalue), Ritz vectors from a twisted factorisation.
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -24,16 +23,10 @@ namespace dss {
 
 constexpr int EIG_THREADS = 512;
 constexpr int EIG_WARPS = EIG_THREADS / 32;
-constexpr bool EIG_PAIR_DEFAULT = false;   // (A/B pending) two 256-thread CTAs per SM when shared memory allows
 constexpr int EIG_MAX_K = 64;
 
 constexpr int EIG_STRIP_CH = 4;                    // float4 column chunks per lane and strip
 constexpr int EIG_STRIP = 32 * 4 * EIG_STRIP_CH;   // 512 columns per strip
-// Up to this N two CTAs (images) could share an SM with the <2, 2> instantiation (64 registers, 2 x 2 loads in flight per
-// lane). Measured on the 296-image step at N = 900 it loses to <4, 1> -- one CTA per SM, 128 registers, all 16 loads of
-// a row group's column blocks in flight per lane: 2.27 ms vs 1.94 ms -- so it is only kept for tuning
-// (DSS_EIG_VARIANT=1).
-constexpr int EIG_SMALL_N = 0;
 
 struct EigParams {
   const float* W;     // [B, N, ldw]
@@ -103,7 +96,9 @@ __host__ __device__ inline size_t eig_double_bytes(int mmax) {
 }
 
 // R = rows per warp and pass of the mat-vec (R independent 128-bit loads in flight per lane), MINB = CTAs per SM the
-// register budget is sized for: <2, 2> for N <= 1024 (two images per SM), <4, 1> beyond.
+// register budget is sized for. The library launches <4, 1, EIG_THREADS>: one CTA per SM, 128 registers, all 16 loads
+// of a row group's column blocks in flight per lane. (Measured on the 296-image step at N = 900: <2, 2, 512>, two
+// images per SM at 64 registers, 2.27 ms vs 1.94 ms; <4, 2, 256> equal, and 3 % slower on the VOC mix.)
 template <int R, int MINB, int NT>
 __global__ void __launch_bounds__(NT, MINB)
 lanczos_laplacian_kernel(EigParams p) {
@@ -563,28 +558,11 @@ static int eig_resolve(int N, int K, int max_steps) {
   return mmax;
 }
 
-// CTAs per SM: 2 when two images' shared memory fits (N <= ~2000) -- the <4, 2, 256> instantiation, two 256-thread CTAs
-// at 128 registers, so that one image's vector phases (reorthogonalisation, Ritz test) overlap the other's mat-vec --
-// else 1 (<4, 1, 512>). DSS_EIG_VARIANT (tuning): 1 forces <2, 2, 512>, 2 forces <4, 1, 512>, 3 forces the pairing.
-static int eig_variant() {
-  static const int variant = [] { const char* e = getenv("DSS_EIG_VARIANT"); return e ? atoi(e) : 0; }();
-  return variant;
-}
-
-static int eig_per_sm(int Npad, int mmax) {
-  const size_t smem = eig_smem_bytes(Npad, mmax);
-  const int fit = (int)((size_t)(220 * 1024) / (smem + 1024));
-  const int v = eig_variant();
-  if (v == 2) return 1;
-  if (v == 1 || v == 3) return fit >= 2 ? 2 : 1;
-  return (EIG_PAIR_DEFAULT && fit >= 2) ? 2 : 1;
-}
-
-static int eig_grid(int B, int Npad, int mmax) {
+// one CTA per image, at most one per SM
+static int eig_grid(int B) {
   int sms = device_sm_count();
   if (sms <= 0) sms = 148;
-  const int g = sms * eig_per_sm(Npad, mmax);
-  return B < g ? B : g;
+  return B < sms ? B : sms;
 }
 
 }  // namespace dss
@@ -595,7 +573,7 @@ extern "C" size_t dss_eigsh_workspace_bytes(int B, int N, int K, int max_steps) 
   if (B <= 0 || N <= 0 || K <= 0) return 0;
   const int Npad = (N + 3) & ~3;
   const int mmax = eig_resolve(N, K, max_steps);
-  const int grid = eig_grid(B, Npad, mmax);
+  const int grid = eig_grid(B);
   const size_t basis = align_up((size_t)grid * (mmax + 1) * Npad * sizeof(float), 256);
   const size_t tri = align_up((size_t)grid * 2 * (K + 1) * mmax * sizeof(double), 256);
   return basis + tri;
@@ -620,7 +598,7 @@ static int eigsh_launch(const float* Wmat, const float* deg, int ldw, int B, int
   p.B = B; p.N = N; p.ldw = ldw; p.Npad = (N + 3) & ~3; p.K = K; p.mode = mode;
   p.mmax = eig_resolve(N, K, max_steps);
   p.tol = tol > 0.f ? tol : 1e-6f;
-  const int grid = eig_grid(B, p.Npad, p.mmax);
+  const int grid = eig_grid(B);
   p.basis = reinterpret_cast<float*>(ws);
   p.tri = reinterpret_cast<double*>(reinterpret_cast<uint8_t*>(ws) +
                                     align_up((size_t)grid * (p.mmax + 1) * p.Npad * sizeof(float), 256));
@@ -629,18 +607,9 @@ static int eigsh_launch(const float* Wmat, const float* deg, int ldw, int B, int
     set_error("eigsh: N=%d with max_steps=%d needs %zu B of shared memory (> 227 KB)", N, p.mmax, smem);
     return DSS_ERR_UNSUPPORTED;
   }
+  DSS_CHECK_CUDA(allow_dynamic_smem(lanczos_laplacian_kernel<4, 1, EIG_THREADS>, (int)smem));
   LaunchScope scope(static_cast<cudaStream_t>(stream), KC_EIGSH);
-  const int per_sm = eig_per_sm(p.Npad, p.mmax);
-  if (per_sm == 2 && eig_variant() == 1) {
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(lanczos_laplacian_kernel<2, 2, EIG_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    lanczos_laplacian_kernel<2, 2, EIG_THREADS><<<grid, EIG_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(p);
-  } else if (per_sm == 2) {
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(lanczos_laplacian_kernel<4, 2, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    lanczos_laplacian_kernel<4, 2, 256><<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(p);
-  } else {
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(lanczos_laplacian_kernel<4, 1, EIG_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    lanczos_laplacian_kernel<4, 1, EIG_THREADS><<<grid, EIG_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(p);
-  }
+  lanczos_laplacian_kernel<4, 1, EIG_THREADS><<<grid, EIG_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(p);
   DSS_CHECK_CUDA(cudaGetLastError());
   return DSS_OK;
 }

@@ -659,8 +659,6 @@ static PFN_encodeTiled get_encode_fn() {
 
 // Tile width used for an N-column GEMM (B operand = weights [N, K]): 256 if it divides N, else 128.
 int gemm_tile_n(int N) {
-  static const char* force = getenv("DSS_GEMM_BN");  // tuning override (experiments only)
-  if (force) return atoi(force);
   // widest tile that divides N: operand bytes per FLOP (shared-memory bandwidth, the binding resource) fall with BN
   return N % 256 == 0 ? 256 : (N % 192 == 0 ? 192 : 128);
 }
@@ -751,12 +749,7 @@ template <int EPI, int BN, int ST = default_stages(BN, epi_uses_tma_store(EPI)),
 static int launch_tc_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmC, int M, int N, int K,
                         const EpiParams& p, cudaStream_t st, int kclass, int batch) {
   using Cfg = TileCfg<BN, epi_uses_tma_store(EPI), ST, CG>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(gemm_f16_tcgen05_kernel<EPI, BN, ST, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        Cfg::SMEM_BYTES));
-    attr_set = true;
-  }
+  DSS_CHECK_CUDA(allow_dynamic_smem(gemm_f16_tcgen05_kernel<EPI, BN, ST, CG>, Cfg::SMEM_BYTES));
   const int pairs_m = cdiv(cdiv(M, BM), 2), tiles_n = cdiv(N, BN);
   int per_img = pairs_m * tiles_n;
   if (p.tri) {   // symmetric output: row pair p visits the n-tiles j >= 2p only (see decode_tile)
@@ -794,15 +787,12 @@ static int launch_tc_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, const CU
 template <int EPI>
 static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmC, int M, int N, int K,
                      const EpiParams& p, cudaStream_t st, int kclass, int bn, int batch = 1) {
-  // CTA-pair MMA (tcgen05.mma.cta_group::2: each CTA holds only its half of the weight tile). Validated on hardware in
-  // round 2 (tests/test_ops_gpu.py under DSS_GEMM_2CTA=1); measured on the 296-image step against the multicast form:
-  // fc2 (K = 1536) 1028 vs 931 TFLOP/s, but qkv / fc1 / proj (K = 384) 844 / 720 / 411 vs 1019 / 760 / 439 -- the
-  // pair's shared accumulator-drain handshake costs more than the halved operand traffic saves when a tile has only
-  // six K slabs. Hence: on for the long-K residual GEMM, off elsewhere; DSS_GEMM_2CTA = 0 / 1 forces it.
-  static const int two_cta_env = [] { const char* e = getenv("DSS_GEMM_2CTA"); return e ? (atoi(e) != 0 ? 1 : 0) : -1; }();
-  const bool two_cta = two_cta_env >= 0 ? two_cta_env == 1 : (EPI == DSS_EPI_BIAS_RESID_F32 && K >= 1024);
-  if constexpr (epi_uses_tma_store(EPI) && EPI != EPI_AFFINITY_F32) {
-    if (two_cta) {
+  // CTA-pair MMA (tcgen05.mma.cta_group::2: each CTA holds only its half of the weight tile), measured on the
+  // 296-image step against the multicast form: fc2 (K = 1536) 1028 vs 931 TFLOP/s, but qkv / fc1 / proj (K = 384)
+  // 844 / 720 / 411 vs 1019 / 760 / 439 -- the pair's shared accumulator-drain handshake costs more than the halved
+  // operand traffic saves when a tile has only six K slabs. Hence: the long-K residual GEMM only.
+  if constexpr (EPI == DSS_EPI_BIAS_RESID_F32) {
+    if (K >= 1024) {
       constexpr int D = 0;   // stage count is derived from the shared-memory budget for CG = 2
       switch (bn) {
         case 128: return launch_tc_bn<EPI, 128, D, 2>(tmA, tmB, tmC, M, N, K, p, st, kclass, batch);
@@ -919,28 +909,5 @@ extern "C" int dss_op_gemm_f16_simt(const void* A, const void* Wt, const float* 
     case DSS_EPI_DROPCLS_F32: return launch_simt<DSS_EPI_DROPCLS_F32>(A, Wt, M, N, K, p, st);
   }
   set_error("gemm: unknown epilogue %d", epilogue);
-  return DSS_ERR_BAD_ARG;
-}
-
-// Tuning probe (not used by the product path): plain bias epilogue with an explicit tile width / ring depth.
-extern "C" int dss_debug_gemm_cfg(const void* A, const void* Wt, const float* bias, void* out, int M, int N, int K,
-                                  int bn, int stages, dss_stream_t stream) {
-  int rc = check_gemm_args(M, N, K, DSS_EPI_BIAS_F16, bias, out, nullptr, 0, 0);
-  if (rc) return rc;
-  CUtensorMap tmA, tmB, tmC;
-  if ((rc = make_tmap_f16(&tmA, A, M, K, BM))) return rc;
-  if ((rc = make_tmap_f16(&tmB, Wt, N, K, bn / 2))) return rc;
-  if ((rc = make_tmap_out(&tmC, out, M, N, 0))) return rc;
-  EpiParams p{out, bias, nullptr, N, 0, 0, 0, nullptr, nullptr, nullptr, 0.f, 0, 0, 0, nullptr, 0};
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int key = bn * 10 + stages;
-  switch (key) {
-    case 1282: return launch_tc_bn<DSS_EPI_BIAS_F16, 128, 2>(tmA, tmB, &tmC, M, N, K, p, st, KC_GEMM_OTHER, 1);
-    case 1283: return launch_tc_bn<DSS_EPI_BIAS_F16, 128, 3>(tmA, tmB, &tmC, M, N, K, p, st, KC_GEMM_OTHER, 1);
-    case 1924: return launch_tc_bn<DSS_EPI_BIAS_F16, 192, 4>(tmA, tmB, &tmC, M, N, K, p, st, KC_GEMM_OTHER, 1);
-    case 2563: return launch_tc_bn<DSS_EPI_BIAS_F16, 256, 3>(tmA, tmB, &tmC, M, N, K, p, st, KC_GEMM_OTHER, 1);
-    case 2564: return launch_tc_bn<DSS_EPI_BIAS_F16, 256, 4>(tmA, tmB, &tmC, M, N, K, p, st, KC_GEMM_OTHER, 1);
-  }
-  set_error("debug_gemm_cfg: unsupported (bn=%d, stages=%d)", bn, stages);
   return DSS_ERR_BAD_ARG;
 }

@@ -76,7 +76,7 @@ __device__ __forceinline__ bool ln_item(int i, int cid, int ncl, int units, int 
 }
 
 // CL = CTAs per cluster: 2 = the pair shares every weight tile by TMA multicast (each CTA loads half), 1 = every CTA
-// loads its own weight tiles (no coupling between CTAs).
+// loads its own weight tiles (no coupling between CTAs). The library launches CL = 2 (DESIGN.md section 9).
 template <bool GELU, int BN, int CL>
 __global__ void __launch_bounds__(LG_THREADS, 1)
 gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC, int pairs,
@@ -408,15 +408,11 @@ gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmB, const __grid
   if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
-template <bool GELU, int BN, int CL>
-static int launch_ln_cl(const CUtensorMap& tmB, const CUtensorMap& tmC, const LnParams& p, cudaStream_t st, int kclass) {
+template <bool GELU, int BN>
+static int launch_ln(const CUtensorMap& tmB, const CUtensorMap& tmC, const LnParams& p, cudaStream_t st, int kclass) {
   using Cfg = LnCfg<BN>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    DSS_CHECK_CUDA(cudaFuncSetAttribute(gemm_ln_f16_tcgen05_kernel<GELU, BN, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        Cfg::SMEM));
-    attr_set = true;
-  }
+  constexpr int CL = 2;
+  DSS_CHECK_CUDA(allow_dynamic_smem(gemm_ln_f16_tcgen05_kernel<GELU, BN, CL>, Cfg::SMEM));
   const int units = cdiv(cdiv(p.M, LG_BM), CL);   // row blocks (CL = 1) or pairs of row blocks (CL = 2)
   int sms = device_sm_count();
   if (sms <= 0) sms = 148;
@@ -439,16 +435,8 @@ static int launch_ln_cl(const CUtensorMap& tmB, const CUtensorMap& tmC, const Ln
   return DSS_OK;
 }
 
-template <bool GELU, int BN>
-static int launch_ln(const CUtensorMap& tmB, const CUtensorMap& tmC, const LnParams& p, cudaStream_t st, int kclass) {
-  static const int cl = [] { const char* e = getenv("DSS_LN_CLUSTER"); return e ? atoi(e) : 2; }();   // tuning (1 | 2)
-  return cl == 1 ? launch_ln_cl<GELU, BN, 1>(tmB, tmC, p, st, kclass) : launch_ln_cl<GELU, BN, 2>(tmB, tmC, p, st, kclass);
-}
-
 // tile width of the fused kernel for an N-column layer (0: not supported)
 int gemm_ln_tile_n(int N) {
-  static const int prefer = [] { const char* e = getenv("DSS_LN_BN"); return e ? atoi(e) : 192; }();   // tuning (128 | 192)
-  if (prefer == 128 && N % 128 == 0) return 128;
   return N % 192 == 0 ? 192 : (N % 128 == 0 ? 128 : 0);
 }
 

@@ -104,7 +104,7 @@ extern "C" int dss_knn_color_counts(const float* rgb, int B, int Hl, int Wl, uin
   DSS_REQUIRE(smem <= 200 * 1024, "knn: N=%d points do not fit in shared memory", N);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DSS_CHECK_CUDA(cudaMemsetAsync(counts, 0, (size_t)B * N * N, st));
-  DSS_CHECK_CUDA(cudaFuncSetAttribute(knn_counts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DSS_CHECK_CUDA(allow_dynamic_smem(knn_counts_kernel, (int)smem));
   dim3 grid(cdiv(N, KNN_WARPS), B);
   const int ks[2] = {20, 10};
   const double ws_[2] = {2.0, 0.1};

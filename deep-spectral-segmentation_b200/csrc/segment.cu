@@ -334,7 +334,7 @@ extern "C" int dss_segment_kmeans(const float* points, long long image_stride, l
   DSS_REQUIRE(smem <= 200 * 1024, "segment_kmeans: %d clusters x %d dims x %d points need %zu B of shared memory", max_clusters,
               dims, N, smem);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DSS_CHECK_CUDA(cudaFuncSetAttribute(kmeans_segment_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DSS_CHECK_CUDA(allow_dynamic_smem(kmeans_segment_kernel, (int)smem));
   int sms = device_sm_count();
   if (sms <= 0) sms = 148;
   const int grid = B < 2 * sms ? B : 2 * sms;

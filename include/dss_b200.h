@@ -133,10 +133,6 @@ int dss_op_gemm_f16(const void* A, const void* Wt, const float* bias, void* out,
 /* Same contract on CUDA cores (slow, fp32 FMA): in-GPU checker for the tensor-core kernel, used by tests only. */
 int dss_op_gemm_f16_simt(const void* A, const void* Wt, const float* bias, void* out, int M, int N, int K,
                          int epilogue, const float* aux, int rin, int rout, dss_stream_t stream);
-/* Tuning probe: dss_op_gemm_f16 with the plain bias->f16 epilogue and an explicit tile width bn in {128,192,256}
- * and TMA ring depth (2..4). Not used by the product path. */
-int dss_debug_gemm_cfg(const void* A, const void* Wt, const float* bias, void* out, int M, int N, int K, int bn,
-                       int stages, dss_stream_t stream);
 /* LayerNorm fused into the GEMM's A-operand producer (the qkv / fc1 layers of ViT-S; K must be 384):
  * out f16 [M, N] = (gelu ? gelu_erf : id)(LayerNorm(x f32 [M, K]; gamma, beta, eps) @ Wt f16 [N, K]^T + bias); N % 128 == 0 */
 int dss_op_gemm_ln_f16(const float* x, const float* gamma, const float* beta, const void* Wt, const float* bias,

@@ -77,6 +77,55 @@ def test_gemm_epilogues(cuda):
     want = torch.full((B, T, d), 3.0, device=cuda)
     want[:, 1:] = accp.view(B, Np, d) + pos[1:]
     assert (xo.view(B, T, d) - want).abs().max().item() <= 2e-4 * accp.abs().max().item()
+    # residual f32 with K >= 1024 (the CTA-pair MMA path), one N per tile width: 128, 192, 256
+    K2 = 1536
+    A2 = torch.randn(M, K2, device=cuda, generator=g).half()
+    for N2 in (128, 384, 768):
+        W2 = (torch.randn(N2, K2, device=cuda, generator=g) * 0.05).half()
+        b2 = torch.randn(N2, device=cuda, generator=g)
+        acc2 = A2.float() @ W2.float().T + b2
+        x = torch.randn(M, N2, device=cuda, generator=g)
+        x0 = x.clone()
+        _gemm(lib, _lib, lib.dss_op_gemm_f16, A2, W2, b2, x, _lib.EPI_BIAS_RESID_F32)
+        assert (x - (x0 + acc2)).abs().max().item() <= 2e-4 * acc2.abs().max().item(), N2
+
+
+def test_gemm_ln_and_attention_on_a_second_device(cuda):
+    """A GEMM, a fused-LayerNorm GEMM and an attention call on cuda:0 and then on cuda:1 in the same process: the
+    launch set-up the library keeps per device (dynamic shared-memory limit, SM count) is in place on both."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two CUDA devices")
+    _lib = load_pkg("_lib"); lib = _lib.load()
+    M, K, N = 300, 384, 1152
+    B, T, heads = 2, 197, 6
+    for dev in (torch.device("cuda:0"), torch.device("cuda:1")):
+        with torch.cuda.device(dev):
+            g = torch.Generator(device=dev).manual_seed(11)
+            st = _lib.stream_ptr(dev)
+            x = torch.randn(M, K, device=dev, generator=g) * 2.0 + 0.5
+            gamma = torch.randn(K, device=dev, generator=g) * 0.5 + 1.0
+            beta = torch.randn(K, device=dev, generator=g) * 0.2
+            Wt = (torch.randn(N, K, device=dev, generator=g) * 0.05).half()
+            bias = torch.randn(N, device=dev, generator=g) * 0.1
+            qkv = (torch.randn(B, T, 3 * heads * 64, device=dev, generator=g) * 1.5).half()
+            A = x.half()
+            out = torch.full((M, N), float("nan"), device=dev)
+            out_ln = torch.full((M, N), float("nan"), device=dev, dtype=torch.float16)
+            att = torch.full((B, T, heads * 64), float("nan"), device=dev, dtype=torch.float16)
+            _lib.check(lib.dss_op_gemm_f16(A.data_ptr(), Wt.data_ptr(), bias.data_ptr(), out.data_ptr(), M, N, K,
+                                           _lib.EPI_BIAS_F32, None, 0, 0, st), "gemm")
+            _lib.check(lib.dss_op_gemm_ln_f16(x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), Wt.data_ptr(), bias.data_ptr(),
+                                              out_ln.data_ptr(), M, N, K, 1e-6, 0, st), "gemm_ln")
+            _lib.check(lib.dss_op_attention_tc_f16(qkv.data_ptr(), att.data_ptr(), B, T, heads, st), "attention")
+            torch.cuda.synchronize(dev)
+            ref = A.float() @ Wt.float().T + bias
+            assert (out - ref).abs().max().item() <= 2e-4 * max(1.0, ref.abs().max().item()), dev
+            xn = torch.nn.functional.layer_norm(x, (K,), gamma, beta, 1e-6)
+            ref = xn.half().float() @ Wt.float().T + bias
+            assert (out_ln.float() - ref).abs().max().item() <= 3e-3 * max(1.0, ref.abs().max().item()), dev
+            q, k, v = qkv.float().view(B, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
+            ref = (((q @ k.transpose(-2, -1)) * 0.125).softmax(-1) @ v).transpose(1, 2).reshape(B, T, heads * 64)
+            assert (att.float() - ref).abs().max().item() <= 4e-3 * max(1.0, ref.abs().max().item()), dev
 
 
 @pytest.mark.parametrize("d", [384, 768])

@@ -1,5 +1,5 @@
-"""Time the tcgen05 attention kernel alone (B x 901 tokens, 6 heads); DSS_ATTN_ABL selects a timing ablation."""
-import importlib, os, sys
+"""Time the tcgen05 attention kernel alone (B x 901 tokens, 6 heads)."""
+import importlib, sys
 from pathlib import Path
 import torch
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
@@ -21,4 +21,4 @@ for _ in range(10):
 ts.sort()
 t = ts[len(ts) // 2]
 flops = 4.0 * B * heads * T * T * 64
-print(f"ABL={os.environ.get('DSS_ATTN_ABL', '0'):>3s} B={B}: {t:.3f} ms  ({t / B * 1024 * 12:.1f} ms per 1024 images x 12 blocks)  {flops / t / 1e9:.0f} TFLOP/s")
+print(f"B={B}: {t:.3f} ms  ({t / B * 1024 * 12:.1f} ms per 1024 images x 12 blocks)  {flops / t / 1e9:.0f} TFLOP/s")

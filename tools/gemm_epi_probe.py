@@ -1,5 +1,4 @@
-"""Times dss_op_gemm_f16 (the product launch path, all epilogues) on the ViT-S shapes of the 256/296-image step.
-Run once plainly and once with DSS_GEMM_2CTA=1 to compare the cta_group::2 path."""
+"""Times dss_op_gemm_f16 (the product launch path, all epilogues) on the ViT-S shapes of the 256/296-image step."""
 import importlib, os, sys
 from pathlib import Path
 import torch
@@ -29,5 +28,5 @@ def run(name, N, K, epi, iters=12):
     if epi == "gelu_f16": ref = torch.nn.functional.gelu(ref)
     err = (out[:512].float() - ref).abs().max().item()
     print(f"{name:5s} N={N:5d} K={K:5d} {epi:9s}: {t*1e3:8.1f} us  {2*M*N*K/t/1e9:8.1f} TFLOP/s  err {err:.2e}", flush=True)
-print("DSS_GEMM_2CTA =", os.environ.get("DSS_GEMM_2CTA"), " M =", M)
+print("M =", M)
 run("qkv", 1152, 384, "bias_f16"); run("fc1", 1536, 384, "gelu_f16"); run("fc2", 384, 1536, "resid_f32"); run("proj", 384, 384, "resid_f32")
