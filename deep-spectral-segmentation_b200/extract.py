@@ -8,7 +8,7 @@
     extract_bbox_features (:500-544)  DINO CLS embedding of every bounding-box crop
 
 Same argument names, defaults, file layouts and skip-if-exists behaviour; all arithmetic runs in libdss_b200. Host I/O
-(decode, pinned staging, .pth / PNG writers) is threaded, see io_pipeline.py."""
+(decode into page-locked batches, .pth / PNG writers) runs on threads and processes, see io_pipeline.py."""
 from __future__ import annotations
 
 from collections import defaultdict
@@ -51,29 +51,41 @@ def _device():
     return torch.device("cuda", torch.cuda.current_device())
 
 
+def _feature_batch(output_dir, files_indices, k: torch.Tensor, model_name, patch_size, H, W, skip=()):
+    """(arrays, items) for io_pipeline's writers: the features dicts of one batch as the reference saves them
+    (extract.py:98-110). k is the batch's (B, N, d) fp32 CPU tensor; shape is the un-cropped image's."""
+    items = [(str(Path(output_dir) / f"{Path(file).stem}.pth"), j,
+              {"file": file, "id": Path(file).stem, "model_name": model_name, "patch_size": patch_size,
+               "shape": (1, 3, H, W)},
+              {"k": ("slice1", "k"), "indices": ("tensor0d", index)})
+             for j, (file, index) in enumerate(files_indices) if j not in skip]
+    return {"k": k.numpy()}, items
+
+
 def _feature_dict(k: torch.Tensor, index: int, file: str, model_name: str, patch_size: int, H: int, W: int) -> dict:
-    """The dict the reference saves at extract.py:98-110 (k is (1, N, d) fp32 on the CPU; shape is un-cropped)."""
-    return {"k": k, "indices": torch.tensor(index), "file": file, "id": Path(file).stem, "model_name": model_name,
-            "patch_size": patch_size, "shape": (1, 3, H, W)}
+    """One features dict (k is (1, N, d)), built as the writers build it."""
+    arrays, (item,) = _feature_batch("", [(file, index)], k, model_name, patch_size, H, W)
+    return io_pipeline._materialise(arrays, *item[1:])
 
 
-def _feature_items(output_dir, files_indices, model_name, patch_size, H, W):
-    """Writer items (io_pipeline) for the feature dicts of one batch: extract.py:98-110, k taken from arrays['k']."""
-    items = []
-    for j, (file, index) in enumerate(files_indices):
-        extra = {"file": file, "id": Path(file).stem, "model_name": model_name, "patch_size": patch_size, "shape": (1, 3, H, W)}
-        items.append((str(Path(output_dir) / f"{Path(file).stem}.pth"), j, extra,
-                      {"k": ("slice1", "k"), "indices": ("tensor0d", index)}))
-    return items
+def _eigs_batch(output_dir, image_ids, evals: torch.Tensor, evecs: torch.Tensor, which_matrix="laplacian", skip=()):
+    """(arrays, items) for the writers: the eigs dicts of one batch (extract.py:242) from the CPU tensors evals [B, K]
+    and evecs [B, K, N]. The 'affinity' branch of the reference keeps `eigenvalues` as the ascending numpy array eigsh
+    returned while the eigenvectors are flipped to descending order (extract.py:171-172); mirrored here."""
+    affinity = which_matrix == "affinity"
+    arrays = {"evals": (evals.flip(1) if affinity else evals).numpy(), "evecs": evecs.numpy()}
+    fields = {"eigenvalues": ("np_slice" if affinity else "slice", "evals"), "eigenvectors": ("slice", "evecs")}
+    return arrays, [(str(Path(output_dir) / f"{image_id}.pth"), j, {}, fields)
+                    for j, image_id in enumerate(image_ids) if j not in skip]
 
 
-def _eigs_items(output_dir, image_ids, which_matrix="laplacian", skip=()):
-    """Writer items for the eigs dicts of one batch (extract.py:242). The 'affinity' branch of the reference keeps
-    `eigenvalues` as the ascending numpy array eigsh returned while the eigenvectors are flipped (extract.py:171-172):
-    the caller passes arrays['evals'] already flipped and it is saved as numpy."""
-    how = "np_slice" if which_matrix == "affinity" else "slice"
-    return [(str(Path(output_dir) / f"{image_id}.pth"), j, {}, {"eigenvalues": (how, "evals"), "eigenvectors": ("slice", "evecs")})
-            for j, image_id in enumerate(image_ids) if j not in skip]
+def _pinned_copy(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    """Starts the device->host copy of t into page-locked memory; read it after the stream has passed this point."""
+    if t is None:
+        return None
+    host = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
+    host.copy_(t, non_blocking=True)
+    return host
 
 
 class _Batcher:
@@ -107,10 +119,51 @@ class _Batcher:
             self._flush(key)
 
 
+def _batch_loop(dataset, todo: List[int], batch_size: int, num_workers: Optional[int], launch):
+    """Runs the images ``todo`` of ``dataset`` through the GPU in batches of one image shape. Decode threads write them
+    straight into page-locked batches (io_pipeline.BatchAssembler). ``launch(batch)`` enqueues the batch's host->device
+    copy, its kernels and the read-back copies, and returns ``finish()``, which hands the results to the writers. A
+    batch is finished only after the NEXT one has been launched, so the GPU works while this thread waits for it.
+    Returns (seconds this thread spent on each activity, the assembler)."""
+    import time
+    tm = dict.fromkeys(("decode_wait", "pinned_alloc", "launch", "wait_gpu", "submit"), 0.0)
+    assembler = io_pipeline.BatchAssembler(dataset.load_raw, todo, max(1, int(batch_size)), num_workers)
+
+    def finish(batch, event, finish_batch):
+        ta = time.perf_counter()
+        event.synchronize()
+        assembler.release(batch)     # its host->device copy is long done: the decode threads may refill it
+        tb = time.perf_counter()
+        finish_batch()
+        tm["wait_gpu"] += tb - ta
+        tm["submit"] += time.perf_counter() - tb
+
+    in_flight = None
+    batches = iter(assembler)
+    while True:
+        ta = time.perf_counter()
+        batch = next(batches, None)
+        tm["decode_wait"] += time.perf_counter() - ta
+        if batch is None:
+            break
+        tb = time.perf_counter()
+        finish_batch = launch(batch)
+        event = torch.cuda.Event()
+        event.record()
+        tm["launch"] += time.perf_counter() - tb
+        if in_flight is not None:
+            finish(*in_flight)
+        in_flight = (batch, event, finish_batch)
+    tm["pinned_alloc"] = assembler.alloc_seconds
+    if in_flight is not None:
+        finish(*in_flight)
+    return tm, assembler
+
+
 def extract_features(images_list: str, images_root: Optional[str], model_name: str, batch_size: int, output_dir: str,
                      which_block: int = -1, checkpoint: Optional[str] = None, seed: Optional[int] = None,
                      random_init: bool = False, yes: Optional[bool] = None, num_workers: Optional[int] = None,
-                     num_workers_out: int = 4, writer: str = "process"):
+                     num_workers_out: int = 4):
     """
     Extract features from a list of images.
 
@@ -132,30 +185,22 @@ def extract_features(images_list: str, images_root: Optional[str], model_name: s
     filenames = Path(images_list).read_text().splitlines()
     dataset = utils.ImagesDataset(filenames=filenames, images_root=images_root)
     print(f"Dataset size: {len(dataset)=}")
-    rings: Dict[tuple, io_pipeline.PinnedRing] = {}
+    todo = []
+    for i in _my_share(list(range(len(dataset)))):
+        output_file = Path(output_dir) / f"{Path(dataset.filenames[i]).stem}.pth"
+        if output_file.is_file():
+            print(f"Skipping existing file {str(output_file)}")
+        else:
+            todo.append(i)
 
-    with io_pipeline.make_writer(writer, num_workers_out) as wr:
-        def flush(shape_key, items):
-            H, W = shape_key
-            ring = rings.get(shape_key)
-            if ring is None:
-                ring = rings[shape_key] = io_pipeline.PinnedRing(shape_key, max(1, int(batch_size)), dev)
-            slot, host = ring.stage([it[0] for it in items])
-            k = model.forward_k(ring.to_device(slot, host), which_block=which_block).cpu()
-            wr.submit_batch({"k": k.numpy()}, _feature_items(output_dir, [(it[1], it[2]) for it in items], model_name,
-                                                             patch_size, H, W))
+    with io_pipeline.make_writer(num_workers_out) as wr:
+        def launch(batch):
+            H, W = batch.key
+            k = model.forward_k(batch.host[:len(batch.items)].to(dev, non_blocking=True), which_block=which_block)
+            k = _pinned_copy(k)
+            return lambda: wr.submit_batch(*_feature_batch(output_dir, batch.items, k, model_name, patch_size, H, W))
 
-        batcher = _Batcher(batch_size, flush)
-        todo = []
-        for i in _my_share(list(range(len(dataset)))):
-            output_file = Path(output_dir) / f"{Path(dataset.filenames[i]).stem}.pth"
-            if output_file.is_file():
-                print(f"Skipping existing file {str(output_file)}")
-            else:
-                todo.append(i)
-        for image, file, index in io_pipeline.ImagePrefetcher(dataset.__getitem__, todo, num_workers):
-            batcher.add((int(image.shape[0]), int(image.shape[1])), (image, file, index))
-        batcher.finish()
+        _batch_loop(dataset, todo, batch_size, num_workers, launch)
     print(f"Saved features to {output_dir}")
 
 
@@ -164,11 +209,6 @@ def _load_image_lr_u8(images_root: str, image_id: str, W_lr: int, H_lr: int) -> 
     from PIL import Image
     image_file = str(Path(images_root) / f"{image_id}.jpg")
     return np.array(Image.open(image_file).resize((W_lr, H_lr), Image.BILINEAR))
-
-
-def _load_image_lr(images_root: str, image_id: str, W_lr: int, H_lr: int) -> np.ndarray:
-    """extract.py:199-204: the low-resolution image / 255 -> float64 (H_lr, W_lr, 3)."""
-    return _load_image_lr_u8(images_root, image_id, W_lr, H_lr) / 255.0
 
 
 def _check_supported(which_matrix, which_color_matrix, image_color_lambda):
@@ -181,12 +221,26 @@ def _check_supported(which_matrix, which_color_matrix, image_color_lambda):
         raise ValueError(f"unknown which_color_matrix={which_color_matrix!r} (the reference knows 'knn' and 'rw')")
 
 
-def _color_inputs(images_root, image_ids, W_lr, H_lr, which_color_matrix, dev):
-    """Low-resolution colour images of a batch on the device: fp32 /255 for 'knn', the uint8 pixels for 'rw'."""
-    lr = np.stack([_load_image_lr_u8(images_root, i, W_lr, H_lr) for i in image_ids]).reshape(len(image_ids), H_lr * W_lr, 3)
-    if which_color_matrix == "rw":
-        return torch.from_numpy(np.ascontiguousarray(lr)).to(dev)
-    return torch.from_numpy((lr / 255.0).astype(np.float32)).to(dev)
+def _laplacian_solver(feats: torch.Tensor, image_ids, lr_size: Tuple[int, int], K, images_root, normalize,
+                      threshold_at_zero, lapnorm, image_color_lambda, which_color_matrix):
+    """``solve(rows, max_steps)`` for a batch of device features [B, N, d]: the which_matrix='laplacian' eigenvalues,
+    eigenvectors and info of every image (rows=None) or of the given batch rows. With image_color_lambda > 0 the colour
+    affinity comes from {images_root}/{image_id}.jpg at lr_size = (H_lr, W_lr), H_lr * W_lr = N: fp32 / 255 for
+    'knn', the uint8 pixels for 'rw'."""
+    rgb_lr = None
+    if image_color_lambda > 0:
+        H_lr, W_lr = lr_size
+        lr = np.stack([_load_image_lr_u8(images_root, i, W_lr, H_lr) for i in image_ids])
+        lr = lr.reshape(len(image_ids), H_lr * W_lr, 3)
+        lr = np.ascontiguousarray(lr) if which_color_matrix == "rw" else (lr / 255.0).astype(np.float32)
+        rgb_lr = torch.from_numpy(lr).to(feats.device)
+
+    def solve(rows, max_steps):
+        f = feats if rows is None else feats[rows]
+        rgb = rgb_lr if (rows is None or rgb_lr is None) else rgb_lr[rows]
+        return spectral.laplacian_eigs(f, K, normalize, threshold_at_zero, lapnorm, rgb, lr_size, image_color_lambda,
+                                       max_steps=max_steps, which_color_matrix=which_color_matrix)[:3]
+    return solve
 
 
 def _bad_rows(evals: torch.Tensor, evecs: torch.Tensor, info: torch.Tensor) -> List[int]:
@@ -201,23 +255,24 @@ def _bad_rows(evals: torch.Tensor, evecs: torch.Tensor, info: torch.Tensor) -> L
     return np.flatnonzero(~ok).tolist()
 
 
-def _solve_with_retry(solve, n_images: int, N: int):
-    """Runs ``solve(sel, max_steps)`` (sel = None for the whole batch, else a list of batch rows) and retries the images
-    whose Lanczos run did not reach its tolerance or came back non-finite with the largest possible Krylov space
-    (max_steps = N - 1). The reference's own safety net is a second eigsh call (which='SM', extract.py:226-234).
-    Returns (eigenvalues, eigenvectors, info, failed rows) on the CPU."""
-    evals, evecs, info = (t.cpu() for t in solve(None, 0))
+def _retry_bad_rows(solve, evals: torch.Tensor, evecs: torch.Tensor, info: torch.Tensor):
+    """Solves again the rows of a batch whose first solve (CPU evals [B, K], evecs [B, K, N], info [B, 4]) did not
+    reach its tolerance or came back non-finite, with the largest possible Krylov space (max_steps = N - 1); the
+    reference's own safety net is a second eigsh call (which='SM', extract.py:226-234). ``solve(rows, max_steps)``
+    returns (eigenvalues, eigenvectors, info) of those rows. A retried row is accepted when it converged and its
+    eigenvalues and eigenvectors are finite; evals / evecs / info are then updated in place.
+    Returns (replaced rows, failed rows, eigenvalues and eigenvectors of the replaced rows as ``solve`` returned them:
+    on its device, None when no row was retried)."""
     bad = _bad_rows(evals, evecs, info)
-    failed = []
-    if bad:
-        ev2, vec2, info2 = (t.cpu() for t in solve(bad, max(N - 1, 1)))
-        for j, i in enumerate(bad):
-            ok = int(info2[j, 1]) == 1 and bool(torch.isfinite(vec2[j]).all() and torch.isfinite(ev2[j]).all())
-            if ok:
-                evals[i], evecs[i], info[i] = ev2[j], vec2[j], info2[j]
-            else:
-                failed.append(i)
-    return evals, evecs, info, failed
+    if not bad:
+        return [], [], None, None
+    ev_d, vec_d, info_d = solve(bad, max(evecs.shape[-1] - 1, 1))
+    ev2, vec2, info2 = ev_d.cpu(), vec_d.cpu(), info_d.cpu()
+    still_bad = set(_bad_rows(ev2, vec2, info2))
+    ok = [j for j in range(len(bad)) if j not in still_bad]
+    replaced = [bad[j] for j in ok]
+    evals[replaced], evecs[replaced], info[replaced] = ev2[ok], vec2[ok], info2[ok]
+    return replaced, [bad[j] for j in sorted(still_bad)], ev_d[ok], vec_d[ok]
 
 
 def _eigs_for_group(data_dicts: List[dict], K: int, images_root, which_features, normalize, lapnorm, threshold_at_zero,
@@ -228,11 +283,10 @@ def _eigs_for_group(data_dicts: List[dict], K: int, images_root, which_features,
     feats = torch.stack([d[which_features].squeeze() for d in data_dicts]).to(torch.float32)
     feats = feats.pin_memory().to(dev, non_blocking=True)
     if which_matrix in ("affinity", "affinity_svd"):
-        def solve(sel, max_steps):
-            f = feats if sel is None else feats[sel]
+        def solve(rows, max_steps):
+            f = feats if rows is None else feats[rows]
             return spectral.affinity_eigs(f, K, which_matrix, normalize, threshold_at_zero, max_steps=max_steps)
     else:
-        rgb_lr, lr_size = None, None
         sizes = utils.get_image_sizes(data_dicts[0])
         P, H_patch, W_patch, H_pad, W_pad = sizes[4:]
         factor = P if image_downsample_factor is None else image_downsample_factor
@@ -243,33 +297,15 @@ def _eigs_for_group(data_dicts: List[dict], K: int, images_root, which_features,
                 feats = spectral.normalize_rows(feats)
                 normalize = False
             feats = spectral.upsample_bilinear(feats, H_patch, W_patch, H_lr, W_lr)
-        if image_color_lambda > 0:
-            rgb_lr = _color_inputs(images_root, [d["file"][:-4] for d in data_dicts], W_lr, H_lr, which_color_matrix, dev)
-            lr_size = (H_lr, W_lr)
-
-        def solve(sel, max_steps):
-            f = feats if sel is None else feats[sel]
-            rgb = rgb_lr if (sel is None or rgb_lr is None) else rgb_lr[sel]
-            return spectral.laplacian_eigs(f, K, normalize, threshold_at_zero, lapnorm, rgb, lr_size, image_color_lambda,
-                                           max_steps=max_steps, which_color_matrix=which_color_matrix)[:3]
-    evals, evecs, info, failed = _solve_with_retry(solve, len(data_dicts), feats.shape[1])
+        solve = _laplacian_solver(feats, [d["file"][:-4] for d in data_dicts], (H_lr, W_lr), K, images_root, normalize,
+                                  threshold_at_zero, lapnorm, image_color_lambda, which_color_matrix)
+    evals, evecs, info = (t.cpu() for t in solve(None, 0))
+    _, failed, _, _ = _retry_bad_rows(solve, evals, evecs, info)
     if failed:
         print(f"Warning: eigensolver did not converge for {[data_dicts[i]['id'] for i in failed]}; no file is written for them")
     if which_matrix == "affinity" and bool((info[:, 2] != 0).any()):
         print("Warning: a negative eigenvalue exceeds the K-th largest in magnitude; eigsh(which='LM') would pick it")
     return evals, evecs, failed
-
-
-def _eigs_dict(which_matrix, evals_k: torch.Tensor, evecs_k: torch.Tensor) -> dict:
-    """extract.py:242. The 'affinity' branch of the reference keeps `eigenvalues` as the ascending numpy array eigsh
-    returned while the eigenvectors are flipped to descending order (extract.py:171-172); mirrored here."""
-    eigenvalues = evals_k.flip(0).numpy().copy() if which_matrix == "affinity" else evals_k.clone()
-    return {"eigenvalues": eigenvalues, "eigenvectors": evecs_k.clone()}
-
-
-def _save_eigs(output_file, which_matrix, evals_k: torch.Tensor, evecs_k: torch.Tensor):
-    Path(output_file).parent.mkdir(parents=True, exist_ok=True)
-    torch.save(_eigs_dict(which_matrix, evals_k, evecs_k), str(output_file))
 
 
 def _extract_eig(inp: Tuple[int, str], K: int, images_root: str, output_dir: str, which_matrix: str = "laplacian",
@@ -290,7 +326,9 @@ def _extract_eig(inp: Tuple[int, str], K: int, images_root: str, output_dir: str
                                            which_matrix, which_color_matrix)
     if failed:
         raise _lib.DssError(f"eigensolver did not converge for {image_id}")
-    _save_eigs(output_file, which_matrix, evals[0], evecs[0])
+    Path(output_file).parent.mkdir(parents=True, exist_ok=True)
+    arrays, (item,) = _eigs_batch(output_dir, [image_id], evals, evecs, which_matrix)
+    io_pipeline.save_item(arrays, item)
 
 
 def extract_eigs(images_root: str, features_dir: str, output_dir: str, which_matrix: str = "laplacian",
@@ -298,7 +336,7 @@ def extract_eigs(images_root: str, features_dir: str, output_dir: str, which_mat
                  threshold_at_zero: bool = True, lapnorm: bool = True, K: int = 20,
                  image_downsample_factor: Optional[int] = None, image_color_lambda: float = 0.0,
                  multiprocessing: int = 0, batch_size: int = 128, yes: Optional[bool] = None,
-                 num_workers: Optional[int] = None, num_workers_out: int = 4, writer: str = "process"):
+                 num_workers: Optional[int] = None, num_workers_out: int = 4):
     """
     Extracts eigenvalues from features.
 
@@ -326,15 +364,14 @@ def extract_eigs(images_root: str, features_dir: str, output_dir: str, which_mat
     start = time.time()
     all_failed: List[str] = []
 
-    with io_pipeline.make_writer(writer, num_workers_out) as wr:
+    with io_pipeline.make_writer(num_workers_out) as wr:
         def flush(key, dds):
             evals, evecs, failed = _eigs_for_group(dds, K, images_root, which_features, normalize, lapnorm,
                                                    threshold_at_zero, image_downsample_factor, image_color_lambda, dev,
                                                    which_matrix, which_color_matrix)
             all_failed.extend(dds[j]["id"] for j in failed)
-            ev = evals.flip(1) if which_matrix == "affinity" else evals
-            wr.submit_batch({"evals": ev.numpy(), "evecs": evecs.numpy()},
-                            _eigs_items(output_dir, [d["file"][:-4] for d in dds], which_matrix, skip=failed))
+            wr.submit_batch(*_eigs_batch(output_dir, [d["file"][:-4] for d in dds], evals, evecs, which_matrix,
+                                         skip=failed))
 
         batcher = _Batcher(batch_size, flush)
         load = lambda i: torch.load(str(inputs[i][1]), map_location="cpu")   # noqa: E731  (file reads overlap on threads)
@@ -516,15 +553,15 @@ def extract_all(images_list: str, images_root: Optional[str], model_name: str, f
                 random_init: bool = False, yes: Optional[bool] = None, single_region_dir: Optional[str] = None,
                 multi_region_dir: Optional[str] = None, non_adaptive_num_segments: int = 4, adaptive: bool = False,
                 infer_bg_index: bool = True, threshold: float = 0.0, num_workers: Optional[int] = None,
-                num_workers_out: int = 4, writer: str = "process"):
+                num_workers_out: int = 4):
     """Fused extract_features + extract_eigs (+ the two segmentation commands): features and eigenvectors never leave
     the GPU between the stages. Writes the eigs files and, if the directories are given, the features files and the
-    single- / multi-region segmentation PNGs, all in the reference's layouts. Decoding, pinned staging and the file
-    writers run on threads (io_pipeline.py)."""
+    single- / multi-region segmentation PNGs, all in the reference's layouts. Decoding and the PNG writers run on
+    threads, the .pth writers in processes (io_pipeline.py)."""
     for dname in (features_dir, eigs_dir, single_region_dir, multi_region_dir):
         if dname:
             utils.make_output_dir(dname, assume_yes=yes)
-    wr = io_pipeline.make_writer(writer, num_workers_out)   # first: writer processes import torch while the model is set up
+    wr = io_pipeline.make_writer(num_workers_out)   # first: writer processes import torch while the model is set up
     model_name = model_name.lower()
     _check_supported("laplacian", which_color_matrix, image_color_lambda)
     dev = _device()
@@ -533,129 +570,71 @@ def extract_all(images_list: str, images_root: Optional[str], model_name: str, f
     filenames = Path(images_list).read_text().splitlines()
     dataset = utils.ImagesDataset(filenames=filenames, images_root=images_root)
     all_failed: List[str] = []
-    decode_threads: dict = {}
     import time
     t_start = time.perf_counter()   # model set-up (weights, packing) is done: what follows is the per-image pipeline
 
-    tm = {"decode_wait": 0.0, "pinned_alloc": 0.0, "launch": 0.0, "wait_gpu": 0.0, "submit": 0.0}
-    in_flight: List[dict] = []       # batches whose kernels / read-back copies are still running (software pipeline)
-    with wr, _png_writer_pool(2) as png_pool:
-        def finish(h):
-            """Second half of a batch: wait for its read-back, retry stragglers, hand everything to the writers."""
-            ta = time.perf_counter()
-            h["event"].synchronize()
-            assembler.release(h["batch"])     # its host->device copy is long done: the decode threads may refill it
-            tb = time.perf_counter()
-            items, H, W, Hp, Wp = h["items"], h["H"], h["W"], h["Hp"], h["Wp"]
-            evals, evecs, info = h["evals"], h["evecs"], h["info"]
-            n_img = len(items)
-            bad = _bad_rows(evals, evecs, info)
-            failed = []
-            if bad:   # rare: largest possible Krylov space for the images that did not reach the tolerance
-                ev2, vec2, info2 = (t.cpu() for t in h["solve"](bad, max(Hp * Wp - 1, 1)))
-                for j, i in enumerate(bad):
-                    if int(info2[j, 1]) == 1 and bool(torch.isfinite(vec2[j]).all()):
-                        evals[i], evecs[i] = ev2[j], vec2[j]
-                    else:
-                        failed.append(i)
-            all_failed.extend(items[j][1] for j in failed)
-            if features_dir:
-                wr.submit_batch({"k": h["k"].numpy()}, [it_ for j, it_ in enumerate(_feature_items(
-                    features_dir, [(it[1], it[2]) for it in items], model_name, patch_size, H, W)) if j not in failed])
-            wr.submit_batch({"evals": evals.numpy(), "evecs": evecs.numpy()},
-                            _eigs_items(eigs_dir, [it[1][:-4] for it in items], skip=failed))
-            for j, (_, file, index) in enumerate(items):
-                if j in failed:
-                    continue
-                if h["masks"] is not None:
-                    png_pool.submit(_save_png, h["masks"][j].numpy().reshape(Hp, Wp).copy(),
-                                    str(Path(single_region_dir) / f"{Path(file).stem}.png"))
-                if h["labels"] is not None:
-                    png_pool.submit(_save_png, h["labels"][j].numpy().reshape(Hp, Wp).copy(),
-                                    str(Path(multi_region_dir) / f"{Path(file).stem}.png"))
-            tm["wait_gpu"] += tb - ta
-            tm["submit"] += time.perf_counter() - tb
-
-        def flush(batch):
-            """First half of a batch: start the H2D copy of the page-locked batch the decode threads filled, enqueue every
-            kernel and the read-back copies; then finish the PREVIOUS batch while this one runs."""
-            H, W = batch.key
-            tb = time.perf_counter()
-            items = [(None, file, index) for file, index in batch.items]
-            host = batch.host[:len(items)]
-            k = model.forward_k(host.to(dev, non_blocking=True), which_block=which_block)
-            Hp, Wp = H // patch_size, W // patch_size
-            rgb_lr, lr_size = None, None
-            if image_color_lambda > 0:
-                rgb_lr = _color_inputs(images_root, [it[1][:-4] for it in items], Wp, Hp, which_color_matrix, dev)
-                lr_size = (Hp, Wp)
-
-            def solve(sel, max_steps):
-                f = k if sel is None else k[sel]
-                rgb = rgb_lr if (sel is None or rgb_lr is None) else rgb_lr[sel]
-                return spectral.laplacian_eigs(f, K, normalize, threshold_at_zero, lapnorm, rgb, lr_size, image_color_lambda,
-                                               max_steps=max_steps, which_color_matrix=which_color_matrix)[:3]
-            evals_d, evecs_d, info_d = solve(None, 0)
-            masks_d = labels_d = None
-            if single_region_dir:
-                masks_d = segment.threshold_masks(evecs_d, threshold, which=1)
-            if multi_region_dir:
-                if adaptive:   # the per-image cluster count comes from the eigenvalues (host arithmetic on K numbers)
-                    ks = [segment.adaptive_num_clusters(e.numpy()) for e in evals_d.cpu()]
-                else:
-                    ks = [non_adaptive_num_segments] * len(items)
-                labels_d = segment.kmeans_labels(evecs_d[:, 1:], ks, (Hp, Wp), infer_bg_index,
-                                                 image_keys=[it[2] for it in items])[0]
-
-            def to_host(t):
-                if t is None:
-                    return None
-                h_ = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
-                h_.copy_(t, non_blocking=True)
-                return h_
-            h = {"items": items, "H": H, "W": W, "Hp": Hp, "Wp": Wp, "solve": solve, "evals": to_host(evals_d),
-                 "evecs": to_host(evecs_d), "info": to_host(info_d), "masks": to_host(masks_d), "labels": to_host(labels_d),
-                 "k": to_host(k) if features_dir else None, "keep": (k, evals_d, evecs_d, info_d, masks_d, labels_d),
-                 "batch": batch}
-            ev = torch.cuda.Event()
-            ev.record(torch.cuda.current_stream(dev))
-            h["event"] = ev
-            tm["launch"] += time.perf_counter() - tb
-            in_flight.append(h)
-            while len(in_flight) > 1:
-                finish(in_flight.pop(0))
-
-        todo = []
-        for i in _my_share(list(range(len(dataset)))):
-            file = dataset.filenames[i]
-            if (Path(eigs_dir) / f"{file[:-4]}.pth").is_file():
-                print(f"Skipping existing file {str(Path(eigs_dir) / (file[:-4] + '.pth'))}")
+    def segment_batch(evals, evecs, keys, grid):
+        """Device masks and K-means labels of a batch (None where no directory asks for them). Cluster counts and
+        generator keys are those of the two segmentation commands, so an image gets the same PNG in any batch."""
+        masks = segment.threshold_masks(evecs, threshold, which=1) if single_region_dir else None
+        labels = None
+        if multi_region_dir:
+            if adaptive:   # the per-image cluster count comes from the eigenvalues (host arithmetic on K numbers)
+                ks = [segment.adaptive_num_clusters(e.numpy()) for e in evals.cpu()]
             else:
-                todo.append(i)
-        # The decode threads group the images by shape and write them straight into page-locked batches
-        # (io_pipeline.BatchAssembler); this thread only sees completed batches.
-        if dataset.transform is None:
-            load = dataset.load_raw
+                ks = [non_adaptive_num_segments] * len(keys)
+            labels = segment.kmeans_labels(evecs[:, 1:], ks, grid, infer_bg_index, image_keys=keys)[0]
+        return masks, labels
+
+    todo = []
+    for i in _my_share(list(range(len(dataset)))):
+        file = dataset.filenames[i]
+        if (Path(eigs_dir) / f"{file[:-4]}.pth").is_file():
+            print(f"Skipping existing file {str(Path(eigs_dir) / (file[:-4] + '.pth'))}")
         else:
-            def load(i):
-                image, file, index = dataset[i]
-                return image.numpy(), False, file, index
-        assembler = io_pipeline.BatchAssembler(load, todo, max(1, int(batch_size)), num_workers)
-        it = iter(assembler)
-        while True:
-            ta = time.perf_counter()
-            batch = next(it, None)
-            tm["decode_wait"] += time.perf_counter() - ta
-            if batch is None:
-                break
-            flush(batch)
-        tm["pinned_alloc"] = assembler.alloc_seconds
-        decode_threads = {k_: round(v_, 3) for k_, v_ in assembler.worker_seconds.items()}
-        decode_threads["threads"] = len(assembler.threads)
-        if assembler.trace is not None:
-            decode_threads["trace"] = [(round(t_ - t_start, 4), ev_, d_) for t_, ev_, d_ in sorted(assembler.trace)]
-        while in_flight:
-            finish(in_flight.pop(0))
+            todo.append(i)
+    with wr, _png_writer_pool(2) as png_pool:
+        def launch(batch):
+            """ViT, eigensolve and segmentations of a batch, and the read-back copies of everything that is written."""
+            H, W = batch.key
+            Hp, Wp = H // patch_size, W // patch_size
+            files, keys = [f for f, _ in batch.items], [i for _, i in batch.items]
+            k = model.forward_k(batch.host[:len(files)].to(dev, non_blocking=True), which_block=which_block)
+            solve = _laplacian_solver(k, [f[:-4] for f in files], (Hp, Wp), K, images_root, normalize, threshold_at_zero,
+                                      lapnorm, image_color_lambda, which_color_matrix)
+            evals_d, evecs_d, info_d = solve(None, 0)
+            masks_d, labels_d = segment_batch(evals_d, evecs_d, keys, (Hp, Wp))
+            evals, evecs, info, masks, labels = map(_pinned_copy, (evals_d, evecs_d, info_d, masks_d, labels_d))
+            k_host = _pinned_copy(k) if features_dir else None
+
+            def finish():
+                """Retry of the images whose solve failed (rare), then everything to the writers."""
+                replaced, failed, ev2, vec2 = _retry_bad_rows(solve, evals, evecs, info)
+                if replaced:   # their PNGs come from the accepted eigenpairs, as in the two segmentation commands
+                    for host, new in zip((masks, labels), segment_batch(ev2, vec2, [keys[j] for j in replaced], (Hp, Wp))):
+                        if new is not None:
+                            host[replaced] = new.cpu()
+                all_failed.extend(files[j] for j in failed)
+                if features_dir:
+                    wr.submit_batch(*_feature_batch(features_dir, batch.items, k_host, model_name, patch_size, H, W,
+                                                    skip=failed))
+                wr.submit_batch(*_eigs_batch(eigs_dir, [f[:-4] for f in files], evals, evecs, skip=failed))
+                for j, file in enumerate(files):
+                    if j in failed:
+                        continue
+                    if masks is not None:
+                        png_pool.submit(_save_png, masks[j].numpy().reshape(Hp, Wp).copy(),
+                                        str(Path(single_region_dir) / f"{Path(file).stem}.png"))
+                    if labels is not None:
+                        png_pool.submit(_save_png, labels[j].numpy().reshape(Hp, Wp).copy(),
+                                        str(Path(multi_region_dir) / f"{Path(file).stem}.png"))
+            return finish
+
+        tm, assembler = _batch_loop(dataset, todo, batch_size, num_workers, launch)
+    decode_threads = {k_: round(v_, 3) for k_, v_ in assembler.worker_seconds.items()}
+    decode_threads["threads"] = len(assembler.threads)
+    if assembler.trace is not None:
+        decode_threads["trace"] = [(round(t_ - t_start, 4), ev_, d_) for t_, ev_, d_ in sorted(assembler.trace)]
     seconds = time.perf_counter() - t_start
     print(f"Saved eigs to {eigs_dir} ({len(todo)} images in {seconds:.2f}s after model set-up: "
           f"{len(todo) / max(seconds, 1e-9):.0f} images/s incl. decode and file writes; main thread: "

@@ -17,23 +17,10 @@ import torch
 from .vit import get_model  # noqa: F401  (re-exported under the reference's name)
 
 
-def read_image_rgb(path) -> np.ndarray:
-    """cv2.imread + BGR->RGB (extract_utils.py:30-31) -> uint8 (H, W, 3). PIL is the fallback decoder."""
-    try:
-        import cv2
-        img = cv2.imread(str(path))
-        if img is None:
-            raise IOError(f"cannot decode {path}")
-        return cv2.cvtColor(img, cv2.COLOR_BGR2RGB)
-    except ImportError:
-        from PIL import Image
-        return np.asarray(Image.open(str(path)).convert("RGB"))
-
-
 def read_image_raw(path):
-    """First half of read_image_rgb: (pixels, is_bgr). The colour swap is left to the caller so that it can write the
-    RGB image straight into a page-locked batch row (io_pipeline.PinnedRing.convert_async) instead of into a temporary
-    that is then copied."""
+    """cv2.imread -> (pixels uint8 (H, W, 3), is_bgr); PIL is the fallback decoder (RGB). The colour swap is left to the
+    caller so that it can write the RGB image straight into a page-locked batch row (io_pipeline.BatchAssembler)
+    instead of into a temporary that is then copied."""
     try:
         import cv2
         img = cv2.imread(str(path))
@@ -43,6 +30,15 @@ def read_image_raw(path):
     except ImportError:
         from PIL import Image
         return np.asarray(Image.open(str(path)).convert("RGB")), False
+
+
+def read_image_rgb(path) -> np.ndarray:
+    """cv2.imread + BGR->RGB (extract_utils.py:30-31) -> uint8 (H, W, 3)."""
+    pixels, is_bgr = read_image_raw(path)
+    if not is_bgr:
+        return pixels
+    import cv2
+    return cv2.cvtColor(pixels, cv2.COLOR_BGR2RGB)
 
 
 class ImagesDataset:

@@ -2,19 +2,17 @@
 (extract/extract.py:60) and writes one .pth per image synchronously (:113, :244); at the rates the kernels run
 (thousands of images per second) both would dominate. Here:
 
-  * ``ImagePrefetcher``  decodes JPEG/PNG files on a thread pool (cv2 / PIL release the GIL while decoding) with a
-                          bounded look-ahead, yielding items in order;
-  * ``PinnedRing``       stages equally shaped uint8 images into a small ring of page-locked batches so that the
-                          host->device copy is asynchronous and the decoder never waits for the GPU;
-  * ``BatchAssembler``   the two steps above in one: decode threads colour-swap each image straight into a row of a
-                          page-locked batch of its shape and hand over completed batches (used by extract_all);
-  * ``AsyncWriter``      runs ``torch.save`` (same dict layouts, so ``torch.load`` consumers are unaffected) on writer
-                          threads; ``close()`` waits for them and re-raises the first error;
-  * ``ProcessWriter``    the same on writer PROCESSES, fed one message per GPU batch: torch.save is ~0.1-0.4 ms of pure
-                          Python per file, and writer threads would take the interpreter lock away from the thread that
-                          feeds the GPU (measured: the main thread spent 1.4 ms per image waiting for the lock).
+  * ``ImagePrefetcher``  runs ``load(i)`` (a file decode or a ``torch.load``) on a thread pool (cv2 / PIL and file
+                          reads release the GIL) with a bounded look-ahead, yielding items in order;
+  * ``BatchAssembler``   decode threads colour-swap each image straight into a row of a page-locked batch of its shape
+                          and hand over completed batches, so that the host->device copy is asynchronous and no staging
+                          copy is made (extract_features, extract_all);
+  * ``ProcessWriter``    runs ``torch.save`` (the reference's dict layouts, so ``torch.load`` consumers are unaffected)
+                          on writer PROCESSES, fed one message per GPU batch: torch.save is ~0.1-0.4 ms of pure Python per
+                          file, and writer threads would take the interpreter lock away from the thread that feeds the GPU
+                          (measured: the main thread spent 1.4 ms per image waiting for the lock).
 
-Pure host code: nothing here touches the device except ``PinnedRing.to_device``'s copy."""
+Pure host code: nothing here touches the device."""
 from __future__ import annotations
 
 import os
@@ -23,7 +21,7 @@ import threading
 from collections import deque
 from concurrent.futures import ThreadPoolExecutor
 from pathlib import Path
-from typing import Callable, Iterable, Iterator, List, Optional, Sequence, Tuple
+from typing import Callable, Iterator, List, Optional, Sequence
 
 import torch
 
@@ -116,90 +114,6 @@ class ImagePrefetcher:
             finally:
                 for f in pending:
                     f.cancel()
-
-
-class PinnedRing:
-    """Ring of page-locked uint8 batches [slots][capacity, H, W, 3] for one image shape. ``stage`` copies decoded images
-    into the next slot (host memcpy), ``to_device`` starts the asynchronous H2D copy and returns the device batch; a
-    slot is reused only after the copy that read it has completed (tracked with a CUDA event)."""
-
-    def __init__(self, shape: Tuple[int, int], capacity: int, device, slots: int = 2, copy_threads: int = 8):
-        H, W = shape
-        self.device = device
-        self.capacity = capacity
-        # torch.empty(pin_memory=True) allocates page-locked memory directly (no pageable copy first)
-        self.bufs = [torch.empty(capacity, H, W, 3, dtype=torch.uint8, pin_memory=True) for _ in range(slots)]
-        self.np_bufs = [b.numpy() for b in self.bufs]    # views of the page-locked memory
-        self.events: List[Optional[torch.cuda.Event]] = [None] * slots
-        self.next = 0
-        copy_threads = int(os.environ.get("DSS_IO_COPY_THREADS", copy_threads))
-        self.copy_threads = copy_threads
-        self._pool = ThreadPoolExecutor(copy_threads, thread_name_prefix="dss-stage") if copy_threads > 1 else None
-
-    def stage(self, images: Sequence[torch.Tensor]) -> Tuple[int, torch.Tensor]:
-        slot = self.next
-        self.next = (self.next + 1) % len(self.bufs)
-        if self.events[slot] is not None:
-            self.events[slot].synchronize()
-        buf = self.bufs[slot][:len(images)]
-        import numpy as np
-        dst = self.np_bufs[slot]
-        # numpy's copy loop releases the interpreter lock (torch's Tensor.copy_ on CPU tensors does not: measured 2.9 GB/s
-        # for the whole staging step with 32 decode threads competing for the lock), so a few threads copy in parallel
-        if self._pool is None or len(images) < 2 * self.copy_threads:
-            for j, im in enumerate(images):
-                np.copyto(dst[j], im.numpy())
-        else:
-            n = self.copy_threads
-
-            def part(t):
-                for j in range(t, len(images), n):
-                    np.copyto(dst[j], images[j].numpy())
-            list(self._pool.map(part, range(n)))
-        return slot, buf
-
-    # ---- incremental staging: the caller assigns (slot, row) as images arrive and the copies run on the pool while it
-    # keeps pulling decoded images; the batch is complete when its futures are
-    def begin(self) -> int:
-        slot = self.next
-        self.next = (self.next + 1) % len(self.bufs)
-        if self.events[slot] is not None:
-            self.events[slot].synchronize()
-        return slot
-
-    def copy_async(self, slot: int, j: int, image: torch.Tensor):
-        import numpy as np
-        dst, src = self.np_bufs[slot][j], image.numpy()
-        if self._pool is None:
-            np.copyto(dst, src)
-            return None
-        return self._pool.submit(np.copyto, dst, src)
-
-    def convert_async(self, slot: int, j: int, pixels, is_bgr: bool):
-        """Like copy_async for a freshly decoded numpy image: a BGR image (cv2.imread) is colour-swapped DIRECTLY into
-        row j of the page-locked batch (one pass over the pixels instead of swap-into-a-temporary + copy)."""
-        import numpy as np
-        dst = self.np_bufs[slot][j]
-
-        def work():
-            if is_bgr:
-                import cv2
-                out = cv2.cvtColor(pixels, cv2.COLOR_BGR2RGB, dst=dst)
-                if out is not dst and not np.shares_memory(out, dst):   # cv2 reallocates when dst does not fit
-                    np.copyto(dst, out)
-            else:
-                np.copyto(dst, pixels)
-        if self._pool is None:
-            work()
-            return None
-        return self._pool.submit(work)
-
-    def to_device(self, slot: int, host_batch: torch.Tensor) -> torch.Tensor:
-        dev = host_batch.to(self.device, non_blocking=True)
-        ev = torch.cuda.Event()
-        ev.record(torch.cuda.current_stream(self.device))
-        self.events[slot] = ev
-        return dev
 
 
 class HostBatch:
@@ -381,71 +295,10 @@ class BatchAssembler:
             self._cv.notify_all()
 
 
-class AsyncWriter:
-    """``submit(obj, path)`` -> ``torch.save(obj, path)`` on one of ``num_threads`` writer threads (bounded queue)."""
-
-    def __init__(self, num_threads: int = 4, max_pending: int = 1024):
-        self.q: "queue.Queue" = queue.Queue(max_pending)
-        self.err: Optional[BaseException] = None
-        self.written = 0
-        self._lock = threading.Lock()
-        self.threads = [threading.Thread(target=self._run, name=f"dss-writer-{i}", daemon=True)
-                        for i in range(max(1, num_threads))]
-        for t in self.threads:
-            t.start()
-
-    def _run(self):
-        while True:
-            item = self.q.get()
-            if item is None:
-                return
-            obj, path = item
-            try:
-                if self.err is None:
-                    Path(path).parent.mkdir(parents=True, exist_ok=True)
-                    tmp = f"{path}.tmp{threading.get_ident()}"
-                    torch.save(obj, tmp)
-                    os.replace(tmp, path)   # a crash never leaves a truncated file for skip-if-exists to trust
-                    with self._lock:
-                        self.written += 1
-            except BaseException as e:  # noqa: BLE001  (reported by close())
-                self.err = e
-
-    def submit(self, obj, path) -> None:
-        if self.err is not None:
-            raise self.err
-        self.q.put((obj, str(path)))
-
-    def submit_batch(self, arrays, items) -> None:
-        """Same interface as ProcessWriter.submit_batch (the dicts are built here, on the calling thread)."""
-        for path, j, extra, fields in items:
-            self.submit(_materialise(arrays, j, extra, fields), path)
-
-    def close(self) -> int:
-        for _ in self.threads:
-            self.q.put(None)
-        for t in self.threads:
-            t.join()
-        if self.err is not None:
-            raise self.err
-        return self.written
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, exc_type, exc, tb):
-        if exc_type is None:
-            self.close()
-        else:   # do not mask the caller's exception
-            try:
-                self.close()
-            except BaseException:  # noqa: BLE001
-                pass
-        return False
-
-
 # ---------------------------------------------------------------------------------------------------------------
-def _materialise(arrays, j, extra, fields):
+def _materialise(arrays, j, extra, fields) -> dict:
+    """The dict of one writer item: ``extra`` plus, for each key of ``fields``, row j of an array of ``arrays`` (see
+    ProcessWriter) or a 0-d tensor."""
     import numpy as np
     obj = dict(extra)
     for key, (how, val) in fields.items():
@@ -462,6 +315,15 @@ def _materialise(arrays, j, extra, fields):
     return obj
 
 
+def save_item(arrays, item) -> None:
+    """torch.save of one writer item (path, row j, extra, fields) to a temporary file that is then renamed to ``path``:
+    a crash never leaves a truncated file for skip-if-exists to trust. The directory must exist."""
+    path, j, extra, fields = item
+    tmp = f"{path}.tmp{os.getpid()}"
+    torch.save(_materialise(arrays, j, extra, fields), tmp)
+    os.replace(tmp, path)
+
+
 def _writer_process_main(q, errq, doneq):
     torch.set_num_threads(1)
     try:
@@ -471,14 +333,12 @@ def _writer_process_main(q, errq, doneq):
                 return
             arrays, items = msg
             made = set()
-            for path, j, extra, fields in items:
-                parent = os.path.dirname(path)
+            for item in items:
+                parent = os.path.dirname(item[0])
                 if parent not in made:      # one mkdir per directory and message, not per file
                     os.makedirs(parent, exist_ok=True)
                     made.add(parent)
-                tmp = f"{path}.tmp{os.getpid()}"
-                torch.save(_materialise(arrays, j, extra, fields), tmp)
-                os.replace(tmp, path)
+                save_item(arrays, item)
             doneq.put(len(items))
     except BaseException as e:  # noqa: BLE001
         import traceback
@@ -491,8 +351,8 @@ class ProcessWriter:
     where fields maps dict keys to ("slice" | "slice1" | "np_slice", array name) or ("tensor0d", int); the worker builds
     each dict and torch.saves it. Started with the 'spawn' method (no fork of a process that holds a CUDA context and
     running threads). Importing torch in the children takes a second or two, so the pool is PERSISTENT: make_writer()
-    hands out the same processes to every command of this interpreter; ``close()`` only waits until everything that
-    was submitted has been written (``flush``)."""
+    hands out the same processes to every command of this interpreter; leaving its ``with`` block only waits until
+    everything that was submitted has been written (``flush``)."""
 
     def __init__(self, num_procs: int = 4, max_pending: int = 16):
         import multiprocessing as mp
@@ -542,9 +402,6 @@ class ProcessWriter:
         self._check()
         return self.done
 
-    def close(self) -> int:
-        return self.flush()
-
     def shutdown(self):
         for _ in self.procs:
             self.q.put(None)
@@ -563,13 +420,9 @@ class ProcessWriter:
 _WRITER_POOL = {}
 
 
-def make_writer(kind: str = "process", workers: int = 4):
-    """'process' (default: writer processes, one message per batch) or 'thread' (torch.save on threads of this process)."""
-    if kind == "process":
-        pool = _WRITER_POOL.get(workers)
-        if pool is None or any(not p_.is_alive() for p_ in pool.procs):
-            pool = _WRITER_POOL[workers] = ProcessWriter(workers)
-        return pool
-    if kind == "thread":
-        return AsyncWriter(workers)
-    raise ValueError(f"unknown writer kind {kind!r}")
+def make_writer(workers: int = 4) -> ProcessWriter:
+    """The persistent ProcessWriter with ``workers`` processes (started on first use, restarted if one has died)."""
+    pool = _WRITER_POOL.get(workers)
+    if pool is None or any(not p_.is_alive() for p_ in pool.procs):
+        pool = _WRITER_POOL[workers] = ProcessWriter(workers)
+    return pool

@@ -1,6 +1,6 @@
 """Batched end-to-end driver of the hot path: uint8 images -> K features -> affinity -> eigenvectors.
 
-Used by extract_all, bench.py and the multi-GPU launcher. Images are the only parallel axis of this workload
+Used by bench.py and the multi-GPU launcher. Images are the only parallel axis of this workload
 (SURVEY 8e): ranks take a strided shard of the image list, the DINO weights are broadcast once from rank 0, and no
 other collective exists on the data path."""
 from __future__ import annotations

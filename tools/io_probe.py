@@ -28,13 +28,13 @@ def main():
     (tmp / "list.txt").write_text("\n".join(names) + "\n")
     (tmp / "warm.txt").write_text("\n".join(names[:128]) + "\n")
     ex.extract_all(str(tmp / "warm.txt"), str(root), "dino_vits16", None, str(tmp / "warm"), K=5, batch_size=128, seed=0)
-    def go(label, batch=128, writer="process", wout=4, **env):
+    def go(label, batch=128, wout=4, **env):
         global run
         run += 1
         old = {k: os.environ.get(k) for k in env}
         os.environ.update({k: str(v) for k, v in env.items()})
         si = float(env.get("SWITCH", 0.005)); sys.setswitchinterval(si)
-        st = ex.extract_all(str(tmp / "list.txt"), str(root), "dino_vits16", None, str(tmp / f"eigs{run}"), K=5, batch_size=batch, seed=0, writer=writer, num_workers_out=wout)
+        st = ex.extract_all(str(tmp / "list.txt"), str(root), "dino_vits16", None, str(tmp / f"eigs{run}"), K=5, batch_size=batch, seed=0, num_workers_out=wout)
         sys.setswitchinterval(0.005)
         for k, v in old.items():
             if v is None: os.environ.pop(k, None)
@@ -112,7 +112,6 @@ def main():
         go("switch0.1ms", SWITCH=0.0001)
         go("batch256", batch=256)
         go("batch64", batch=64)
-        go("threadwriter", writer="thread")
     # decode only
     ds = ex.utils.ImagesDataset(names, str(root))
     for w in (16, 32, 64):
